@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- MPGP iterations/second on the named configurations (BASELINE.json), one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload auto|c3|c2|c2x|c2r|c5|c4|...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload auto|c3|c2|c2x|c2r|c5|c4|...] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" is ONE MPGP iteration (SpMV + fused update + direction update, src/qps/impls/mpgp/mpgp.c:511-641) of a
@@ -21,6 +21,11 @@ QPSSolve that runs through the C ABI of libpermon_b200.so.  W warm-up iterations
 The headline workload is the SAME at every N: C3 (3-D obstacle 512^3, 134 M dofs, z-slab row partition, strong scaling).
 The N = 1 line additionally carries C2 (2-D obstacle 4096^2, 16.7 M dofs) as a nested `c2` object with its own
 roofline / e2e / parity / cpu_baseline.
+
+--dump-outputs DIR writes the iterate x the timed window ended with (what QPSSolve hands back to its caller) as
+DIR/<workload>_x.npy in float64, one file per measured workload: every entry up to DUMP_MAX entries, beyond that the
+entries at dump_index(n), a fixed seeded sample of global row numbers.  The inputs are generated from fixed seeds, so
+two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -70,6 +75,30 @@ WORKLOADS = {
     "t2d": dict(kind="2d", N=512, bscale=-30.0, label="tiny 2-D obstacle 512^2 (harness self-test)"),
     "t3d": dict(kind="3d", N=64, label="tiny 3-D obstacle 64^3 (harness self-test)"),
 }
+
+
+DUMP_MAX = 1 << 21      # entries per dumped array: 16 MB in float64, so that the C3 + C2 line stays under 64 MB
+
+
+def dump_index(n):
+    """the global rows of an n-vector that --dump-outputs writes: all of them up to DUMP_MAX, else a fixed seeded sample, sorted"""
+    if n <= DUMP_MAX:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_MAX, replace=False))
+
+
+def owned_sample(x_loc, r0, idx):
+    """entries of the global sample idx held by this rank's rows [r0, r0 + len(x_loc)), 0 at the others: summed over the ranks it is x[idx],
+    exactly (every entry has one owner)"""
+    own = (idx >= r0) & (idx < r0 + len(x_loc))
+    out = x_loc.new_zeros(len(idx))
+    out[own] = x_loc[idx[own] - r0]
+    return out
+
+
+def dump(dump_dir, name, x):
+    os.makedirs(dump_dir, exist_ok=True)
+    np.save(os.path.join(dump_dir, f"{name}_x.npy"), np.asarray(x, dtype=np.float64))
 
 
 def workload_spec(name):
@@ -279,7 +308,7 @@ class Env:
     pass
 
 
-def measure(env, spec, K, W, want_e2e=True, want_cpu=True, want_parity=True, cpu_budget=20.0, sampler=None):
+def measure(env, spec, K, W, want_e2e=True, want_cpu=True, want_parity=True, cpu_budget=20.0, sampler=None, dump_dir=None):
     P, torch, dev, stream, rank, size = env.P, env.torch, env.dev, env.stream, env.rank, env.size
     dist = env.dist
 
@@ -378,6 +407,13 @@ def measure(env, spec, K, W, want_e2e=True, want_cpu=True, want_parity=True, cpu
     c_all = P.QPSMPGPGetStepCounts(h["qps"])
     counts = {k: c_all[k] - c_warm[k] for k in c_all}
     value = K / (ms * 1e-3)
+    if dump_dir:
+        x_dump = owned_sample(h["dev"]["x"], pr.r0, torch.from_numpy(dump_index(n_glob)).to(dev))
+        if size > 1:
+            dist.all_reduce(x_dump)
+        if rank == 0:
+            dump(dump_dir, spec["name"], x_dump.cpu().numpy())
+        del x_dump
 
     # ---------------- roofline: every fused kernel timed per launch in a repeat of the timed region ----------
     h["dev"]["x"].copy_(x_after_warmup)
@@ -537,7 +573,7 @@ def measure(env, spec, K, W, want_e2e=True, want_cpu=True, want_parity=True, cpu
 # ----------------------------------------------------------------------------------------------------------
 # C4: SVM dual through SMALXE + MPGP, Hessian applied as two long-row SpMVs (BASELINE.json configs[3])
 # ----------------------------------------------------------------------------------------------------------
-def measure_c4(env, n, K, W, want_cpu=True, want_parity=True):
+def measure_c4(env, n, K, W, want_cpu=True, want_parity=True, dump_dir=None):
     """min 1/2 a'(Z Z')a - 1'a, 0 <= a <= 1, y'a = 0; Z = diag(y) X, X n x n with n/1000 (at most 1000) non-zeros per row.  A step is one
     INNER MPGP iteration of a bounded SMALXE window (1 outer iteration, K inner iterations; at n = d the dual is too ill-conditioned to
     converge inside any bench window, in the oracle as well).  The dominant kernel is the long-row SpMV pair of the Hessian."""
@@ -616,6 +652,9 @@ def measure_c4(env, n, K, W, want_cpu=True, want_parity=True):
     its = P.QPSSMALXEGetStatistics(h["qps"])["inner_iter_accu"]
     counts = P.QPSMPGPGetStepCounts(inner)
     value = its / (ms * 1e-3)
+    if dump_dir:
+        P.VecSyncToHost(h["x"])
+        dump(dump_dir, "c4", h["xh"][dump_index(n)])
     destroy(h)
     torch.cuda.empty_cache()
     # ---- e2e: host arrays -> upload (+ tile-ELL re-layout on the device) -> set-up (two power methods) -> K inner iterations -> download
@@ -684,6 +723,7 @@ def main():
     ap.add_argument("--no-c2", action="store_true", help="N = 1, workload auto: skip the nested C2 object")
     ap.add_argument("--cpu-budget", type=float, default=20.0)
     ap.add_argument("--c4-n", type=int, default=1_000_000, help="--workload c4: rows = columns of X (BASELINE config 4: 1M)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the iterate of the timed window's last step as DIR/<workload>_x.npy")
     args = ap.parse_args()
     K, W = max(1, args.steps), max(3, args.warmup)
     rank = int(os.environ.get("RANK", "0"))
@@ -692,15 +732,18 @@ def main():
     spec = workload_spec(args.workload if args.workload != "c4" else "c3")
 
     if args.impl == "reference":
-        # the reference's own CPU implementation cannot be built here (PETSc/MPI absent): time the oracle port on all host cores.
-        # A bounded sample of the same workload: min(K, what ~60 s of CPU time allow) iterations from x0, iteration loop timed.
+        # the reference's own CPU implementation needs PETSc + MPI: time the oracle port on all host cores, with the protocol of the GPU arm --
+        # W warm-up iterations from x0, then exactly K timed iterations of a new solve from that iterate, the power method's estimate reused
         if rank != 0:
             return
         pr = generate(spec, 0, 1)
-        Kp = oracle_sample_size(pr.N, pr.nnz, K, 60.0)
-        _, res = oracle_window(pr, Kp)
-        sample = (f"{res['its']} MPGP iterations from x0 of the full-size workload ({pr.N} dofs), {res['threads']} OpenMP threads standing in for MPI ranks; "
-                  "iteration loop timed, power-method set-up outside")
+        pr.x0, res_w = oracle_window(pr, W)
+        x, res = oracle_window(pr, K, maxeig=res_w["maxeig"])
+        assert (res_w["its"], res["its"]) == (W, K), (res_w["its"], res["its"], W, K)
+        if args.dump_outputs:
+            dump(args.dump_outputs, spec["name"], x[dump_index(pr.N)])
+        sample = (f"{res['its']} MPGP iterations after {W} warm-up iterations from x0 of the full-size workload ({pr.N} dofs), {res['threads']} OpenMP "
+                  "threads standing in for MPI ranks; iteration loop timed, power-method set-up outside")
         line = dict(metric=METRIC, value=res["value"], unit=UNIT, n_gpus=args.gpus, steps=K, warmup=W, ms_per_step=1e3 / res["value"],
                     higher_is_better=True, scaling="strong", vs_baseline=None, dtype="f64", data="synthetic", impl="reference",
                     config=dict(workload=spec["label"], n=int(pr.N), nnz=int(pr.nnz), l2=L2_NOTE),
@@ -747,21 +790,21 @@ def main():
     sampler.start()
     if args.workload == "c4":
         assert size == 1, "the C4 product operator is single-GPU"
-        res = measure_c4(env, args.c4_n, K, W, want_cpu=not args.no_cpu_baseline, want_parity=not args.no_parity)
+        res = measure_c4(env, args.c4_n, K, W, want_cpu=not args.no_cpu_baseline, want_parity=not args.no_parity, dump_dir=args.dump_outputs)
         line = dict(metric=METRIC, value=res["value"], unit=UNIT, n_gpus=1, steps=res["steps"], warmup=W, ms_per_step=res["ms_per_step"], higher_is_better=True,
                     scaling="strong", vs_baseline=None, dtype="f64", data="synthetic", config=res["config"], details=res["details"], clocks=sampler.stop(),
                     e2e=res["e2e"], gpu_launches=res["gpu_launches"], roofline=res["roofline"], cpu_baseline=res["cpu_baseline"], parity=res["parity"])
         print(json.dumps(line), flush=True)
         return
     res = measure(env, spec, K, W, want_e2e=not args.no_e2e, want_cpu=not args.no_cpu_baseline, want_parity=not args.no_parity,
-                  cpu_budget=args.cpu_budget, sampler=sampler)
+                  cpu_budget=args.cpu_budget, sampler=sampler, dump_dir=args.dump_outputs)
     clocks = sampler.stop()
 
     c2 = None
     if size == 1 and args.workload == "auto" and not args.no_c2:
         # BASELINE.json also quotes the metric on C2 (16.7M dofs, one GPU): same legs, nested
         c2 = measure(env, workload_spec("c2"), K, W, want_e2e=not args.no_e2e, want_cpu=not args.no_cpu_baseline, want_parity=not args.no_parity,
-                     cpu_budget=min(args.cpu_budget, 10.0))
+                     cpu_budget=min(args.cpu_budget, 10.0), dump_dir=args.dump_outputs)
         c2["note"] = "C2 = BASELINE.json configs[1] (the 16.7M-dof single-GPU case); the headline workload of this line is C3 so that the --gpus N series is one workload"
 
     if rank == 0:
