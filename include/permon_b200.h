@@ -214,6 +214,34 @@ PERMON_EXTERN PetscErrorCode MatB200GetHostSplit(Mat A, const PetscInt **dia, co
    stream_bytes = bytes one SpMV reads for the matrix itself (diagonal + off-diagonal block); coded_tiles / tiles of the packed form.
    Uploads a row-partitioned matrix if it is not on the device yet. */
 PERMON_EXTERN PetscErrorCode MatB200GetStorageInfo(Mat A, PetscInt *kind, PetscReal *stream_bytes, PetscInt *coded_tiles, PetscInt *tiles);
+/* like MatCreateMPIAIJWithArrays, but di / dj / da are CUDA device pointers (int32 row pointer, GLOBAL column ids, fp64 values) of the
+   device the library runs on.  The arrays must be complete when the call is made (device-synchronised, or written on the stream of
+   PermonB200GetStream).  The matrix is re-coded on the GPU into the same stored form the host constructor builds; the call returns when
+   the arrays are no longer read, and nothing of them is kept (the caller may free or overwrite them).  Null arrays: PETSC_ERR_ARG_NULL;
+   host memory: PETSC_ERR_ARG_WRONG. */
+PERMON_EXTERN PetscErrorCode MatB200CreateAIJWithDeviceArrays(MPI_Comm comm, PetscInt m, PetscInt n, PetscInt M, PetscInt N, const PetscInt di[], const PetscInt dj[],
+                                                              const PetscScalar da[], Mat *mat);
+/* parts of the stored form of an AIJ matrix (MatB200GetStoredForm): field + MATB200_FORM_OFFDIAG selects the off-diagonal block of a
+   row-partitioned matrix instead of the diagonal block (the whole matrix on one rank) */
+#define MATB200_FORM_SCALARS 0   /* 15 int64: kind, n, ncols, nnz, st_npat, st_nwin, st_lmax, st_dlo, st_dhi, pk_max, pk_bytes, pk_coded, stages, tile_cap, W */
+#define MATB200_FORM_ST_MASKS 1  /* all-stencil form: presence byte per row (ntiles * 256) */
+#define MATB200_FORM_ST_PID 2    /* pattern id per tile */
+#define MATB200_FORM_ST_PATS 3   /* pattern table */
+#define MATB200_FORM_PK_BLOB 4   /* packed tiles: blob (incl. its 16 trailing bytes) */
+#define MATB200_FORM_PK_OFF 5    /* tile offsets in 16-byte units (ntiles + 1) */
+#define MATB200_FORM_CSR_IA 6
+#define MATB200_FORM_CSR_JA 7    /* up to nnz */
+#define MATB200_FORM_CSR_A 8     /* up to nnz */
+#define MATB200_FORM_ELL_VAL 9   /* tile-ELL arrays */
+#define MATB200_FORM_ELL_COL 10
+#define MATB200_FORM_ELL_LEN 11
+#define MATB200_FORM_ELL_LT 12
+#define MATB200_FORM_ELL_OFF 13
+#define MATB200_FORM_ROWS 14     /* row id of every compressed row (off-diagonal block) */
+#define MATB200_FORM_OFFDIAG 16
+/* copy one part of the stored form into a host buffer of *nbytes bytes; buf == NULL returns the size of the part in *nbytes (0: the
+   matrix has no such array).  Uploads a row-partitioned matrix if it is not on the device yet. */
+PERMON_EXTERN PetscErrorCode MatB200GetStoredForm(Mat A, PetscInt part, void *buf, size_t *nbytes);
 /* host-side packer of the device matrix format (permon_b200/csrc/pack.cpp), exposed so that the format can be checked without a
    GPU: tile t occupies blob[16*tile_off[t] .. 16*tile_off[t+1]).  *blob == NULL when the matrix cannot be packed. */
 PERMON_EXTERN PetscErrorCode PermonB200PackTiles(PetscInt n, const PetscInt ia[], const PetscInt ja[], const PetscScalar a[], unsigned char **blob,

@@ -353,6 +353,47 @@ def MatCreateAIJFromDevicePointers(m, n, dia, dja, da, keep=None, comm=None):
     return A
 
 
+def MatCreateAIJFromDeviceTensors(ia, ja, a, ncols_local=None, comm=None):
+    """MatB200CreateAIJWithDeviceArrays: local rows in CSR with GLOBAL column indices, as torch CUDA tensors (int32 / int32 / float64,
+    contiguous) on the library's device.  The matrix is re-coded on the GPU into the form MatCreateAIJ builds; the tensors are not kept
+    and may be freed or overwritten when the call returns."""
+    import torch
+    for t, dt, name in ((ia, torch.int32, "ia"), (ja, torch.int32, "ja"), (a, torch.float64, "a")):
+        if not isinstance(t, torch.Tensor) or t.device.type != "cuda":
+            raise TypeError(f"{name}: a torch CUDA tensor is required")
+        if t.dtype != dt or not t.is_contiguous() or t.dim() != 1:
+            raise TypeError(f"{name}: a contiguous 1-D {dt} tensor is required (got {t.dtype}, shape {tuple(t.shape)})")
+    m = ia.numel() - 1
+    n = m if ncols_local is None else ncols_local
+    # the tensors were written on torch's current stream: the library reads them on its own stream
+    torch.cuda.current_stream(ia.device).synchronize()
+    A = C.c_void_p()
+    call("MatB200CreateAIJWithDeviceArrays", comm or world(), C.c_int(m), C.c_int(n), C.c_int(DECIDE), C.c_int(DECIDE),
+         C.c_void_p(ia.data_ptr()), C.c_void_p(ja.data_ptr() if ja.numel() else None), C.c_void_p(a.data_ptr() if a.numel() else None), C.byref(A))
+    return A
+
+
+FORM_PARTS = {"scalars": 0, "st_masks": 1, "st_pid": 2, "st_pats": 3, "pk_blob": 4, "pk_off": 5, "csr_ia": 6, "csr_ja": 7, "csr_a": 8,
+              "ell_val": 9, "ell_col": 10, "ell_len": 11, "ell_lt": 12, "ell_off": 13, "rows": 14}
+FORM_OFFDIAG = 16
+FORM_SCALARS = ("kind", "n", "ncols", "nnz", "st_npat", "st_nwin", "st_lmax", "st_dlo", "st_dhi", "pk_max", "pk_bytes", "pk_coded", "stages",
+                "tile_cap", "W")
+
+
+def MatGetStoredForm(A, offdiag=False):
+    """MatB200GetStoredForm: every part of the stored form of the diagonal (or off-diagonal) block as bytes, plus the scalar fields"""
+    out = {}
+    for name, part in FORM_PARTS.items():
+        part += FORM_OFFDIAG if offdiag else 0
+        nb = C.c_size_t()
+        call("MatB200GetStoredForm", A, C.c_int(part), None, C.byref(nb))
+        buf = C.create_string_buffer(max(nb.value, 1))
+        call("MatB200GetStoredForm", A, C.c_int(part), buf, C.byref(nb))
+        out[name] = buf.raw[:nb.value]
+    out["fields"] = dict(zip(FORM_SCALARS, np.frombuffer(out["scalars"], dtype=np.int64).tolist()))
+    return out
+
+
 def MatCreateOneRow(vec):
     A = C.c_void_p()
     call("MatCreateOneRow", vec, C.byref(A))
@@ -699,10 +740,25 @@ class Solved:
     pass
 
 
-def solve_problem(pr, qps_type=None, options: str = "", monitor=None, keep=False, device_arrays=None):
+def solve_problem(pr, qps_type=None, options: str = "", monitor=None, keep=False, device_arrays=None, device_input=None):
     """Build QP + QPS for a permon_b200.problems.QPProblem through the C ABI, solve, return a result object.
 
-    `options` is a PETSc-style option string ("-qps_rtol 1e-8 -qps_mpgp_expansion_type gf ...")."""
+    `options` is a PETSc-style option string ("-qps_rtol 1e-8 -qps_mpgp_expansion_type gf ...").
+    `device_input`: "keep" builds the AIJ matrices from torch CUDA tensors (MatCreateAIJFromDeviceTensors), "zero" does the same and
+    zeroes the tensors right after each constructor returns."""
+    if device_input:
+        import torch
+
+        def MatCreateAIJ(ia, ja, a, ncols_local=None):
+            t = [torch.as_tensor(np.ascontiguousarray(v, dtype=dt)).cuda() for v, dt in ((ia, np.int32), (ja, np.int32), (a, np.float64))]
+            M = MatCreateAIJFromDeviceTensors(*t, ncols_local=ncols_local)
+            if device_input == "zero":
+                for v in t:
+                    v.zero_()
+                torch.cuda.synchronize()
+            return M
+    else:
+        MatCreateAIJ = globals()["MatCreateAIJ"]
     options_clear()
     if options:
         call("PetscOptionsInsertString", None, options.encode())

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "csrc", "build")
 LIB = os.path.join(HERE, "libpermon_b200.so")
-SOURCES = ["kernels.cu", "shim.cpp", "qp.cpp", "qps.cpp", "pack.cpp", "qps_lin.cpp"]
+SOURCES = ["kernels.cu", "shim.cpp", "qp.cpp", "qps.cpp", "pack.cpp", "qps_lin.cpp", "recode.cu"]
 HEADERS = ["device.h", "mpgp_ctl.h", "objects.h", os.path.join("..", "..", "include", "permon_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]

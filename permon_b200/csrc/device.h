@@ -124,6 +124,22 @@ struct RawBuf {
   size_t         size() const { return n; }
 };
 
+// blob bytes of one tile of each kind (pack.cpp); shared by the host builder and the device re-coder (recode.cu)
+__host__ __device__ inline size_t pk_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+__host__ __device__ inline size_t pk_coded_bytes(int ndict, int nrows, int nnz, bool uniform)
+{
+  size_t b = sizeof(PkHeader) + pk_up(ndict, 2) * 8 + pk_up(ndict, 4) * 4;
+  if (!uniform) b += pk_up((size_t)nrows + 1, 8) * 2;
+  b += pk_up(nnz, 16);
+  return pk_up(b, 16);
+}
+__host__ __device__ inline size_t pk_stencil_bytes(int L, int nrows) { return pk_up(sizeof(PkHeader) + pk_up(L, 2) * 8 + pk_up(L, 4) * 4 + pk_up((size_t)nrows, 16), 16); }
+__host__ __device__ inline size_t pk_raw_bytes(int nrows, int nnz)
+{
+  return pk_up(sizeof(PkHeader) + pk_up(nnz, 2) * 8 + pk_up(nnz, 4) * 4 + pk_up((size_t)nrows + 1, 8) * 2, 16);
+}
+int pattern_windows(StPattern &P);   // lays out the x windows of a pattern; returns the last window index
+
 struct StencilHost {   // host side of the all-stencil form, filled by pk_build
   bool                       valid = false;
   std::vector<StPattern>     pats;
@@ -324,8 +340,26 @@ int k_ctrl_B(MpgpCtl *S, const double *rb);
 int k_pack(int n, const int *idx, const double *x, double *buf);
 
 double csr_stream_bytes(const CsrDev &A);   // bytes one SpMV must read for the matrix itself (CSR: 12 nnz + 4(n+1); packed: blob + directory)
-int  spmv_config(CsrDev &A, const int *h_ia);   // picks kind / W / grid from the host row pointer
+int  spmv_config(CsrDev &A, const int *h_ia);   // picks kind / W / grid from the host row pointer (spmv_stats + spmv_decide)
+void spmv_stats(int n, const int *h_ia, int *maxrow, int *tile_cap);   // longest row, most non-zeros of a 256-row tile
+void spmv_decide(CsrDev &A, int maxrow, int tile_cap);                  // the kernel flavour from those statistics and A.nnz
 int  csr_to_tile_ell(CsrDev &A, const int *h_ia);   // long-row matrices: re-lay the uploaded CSR out as tile-ELL (kind 5) on the device
+int  csr_to_tile_ell_widths(CsrDev &A, const std::vector<int> &tile_maxrow);   // same, from the longest row of every tile
+// all-stencil form (kind 4) on the device: sets the scalar fields of A from the pattern table (upload_stencil, recode.cu)
+void stencil_set_fields(CsrDev &A, const std::vector<StPattern> &pats, int nwin, size_t masks_bytes, size_t npid);
+// device re-coder (recode.cu): the stored form upload_csr builds from a host CSR, built on the device from a device CSR (int32
+// row pointer, column ids in [0, ncols), fp64 values).  The caller's arrays are only read, unless own_ia / own_ja / own_a are given:
+// library-owned arrays padded like upload_csr's (8 zero elements behind each) that a matrix staying CSR adopts (the pointers are then
+// set to NULL; whatever is left non-NULL still belongs to the caller)
+int  recode_csr_dev(CsrDev &A, int nrows, int ncols, const int *d_ia, const int *d_ja, const double *d_a, int **own_ia = nullptr, int **own_ja = nullptr,
+                    double **own_a = nullptr);
+// all-stencil form of the diagonal block [c0, c0 + ncols) of a row-partitioned device CSR with GLOBAL columns, straight from the caller's
+// arrays (pk_stencil_windowed); *done = false when some tile is not a stencil tile or there are too many patterns
+int  recode_stencil_window_dev(CsrDev &A, int m, const int *d_ia, const int *d_ja, const double *d_a, int c0, int ncols, bool *done);
+// row-partitioned device CSR with GLOBAL columns: the ghost entries (row, global column, value) in storage order on the host and, with
+// want_diag, the diagonal block [c0, c0 + ncols) as a padded device CSR with local columns (library-owned, released with dfree)
+int  split_rows_dev(int m, const int *d_ia, const int *d_ja, const double *d_a, int c0, int ncols, bool want_diag, int **dia, int **dja, double **da,
+                    OffDiagEntries &off);
 int  elementwise_grid();
 int  fused_C_grid(int n);   // CTAs of K_C for n local rows (K_A adds that many partial sums of g.p)
 int  max_red_blocks();

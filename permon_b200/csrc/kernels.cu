@@ -1647,17 +1647,26 @@ __global__ void __launch_bounds__(NT) k_csr_to_ell(int n, const int *__restrict_
 }
 int csr_to_tile_ell(CsrDev &A, const int *h_ia)
 {
+  const int        ntiles = (A.n + TR - 1) / TR;
+  std::vector<int> maxrow((size_t)ntiles);
+  for (int t = 0; t < ntiles; t++) {
+    int L = 0;
+    for (int r = t * TR; r < std::min(A.n, (t + 1) * TR); r++) L = std::max(L, h_ia[r + 1] - h_ia[r]);
+    maxrow[t] = L;
+  }
+  return csr_to_tile_ell_widths(A, maxrow);
+}
+int csr_to_tile_ell_widths(CsrDev &A, const std::vector<int> &tile_maxrow)
+{
   const int ntiles = (A.n + TR - 1) / TR;
   if (ntiles == 0 || !A.ia || !A.ja || !A.a) return 0;
   std::vector<int64_t> off((size_t)ntiles);
   std::vector<int>     lt((size_t)ntiles);
   int64_t              tot = 0;
   for (int t = 0; t < ntiles; t++) {
-    int L = 0;
-    for (int r = t * TR; r < std::min(A.n, (t + 1) * TR); r++) L = std::max(L, h_ia[r + 1] - h_ia[r]);
-    L      = (L + ELL_U - 1) / ELL_U * ELL_U;
-    lt[t]  = L;
-    off[t] = tot;
+    const int L = (tile_maxrow[t] + ELL_U - 1) / ELL_U * ELL_U;
+    lt[t]       = L;
+    off[t]      = tot;
     tot += (int64_t)L * TR;
   }
   if (tot > (int64_t)(1.3 * (double)A.nnz) + 65536) return 0;   // ragged rows: the padding would cost more than it saves
@@ -1974,11 +1983,10 @@ double csr_stream_bytes(const CsrDev &A)
   return 12.0 * (double)A.nnz + 4.0 * (A.n + 1);
 }
 
-// decide the kernel flavour from the row pointer (host copy)
-int spmv_config(CsrDev &A, const int *h_ia)
+// decide the kernel flavour from the row pointer (host copy); the device re-coder computes the same statistics on the device
+void spmv_stats(int n, const int *h_ia, int *maxrow_out, int *cap_out)
 {
-  const int n = A.n;
-  int       maxrow = 0, cap = 0;
+  int maxrow = 0, cap = 0;
   for (int r0 = 0; r0 < n; r0 += TR) {
     int r1 = (r0 + TR < n) ? r0 + TR : n;
     int t  = h_ia[r1] - h_ia[r0];
@@ -1989,6 +1997,19 @@ int spmv_config(CsrDev &A, const int *h_ia)
     int l = h_ia[r + 1] - h_ia[r];
     if (l > maxrow) maxrow = l;
   }
+  *maxrow_out = maxrow;
+  *cap_out    = cap;
+}
+int spmv_config(CsrDev &A, const int *h_ia)
+{
+  int maxrow, cap;
+  spmv_stats(A.n, h_ia, &maxrow, &cap);
+  spmv_decide(A, maxrow, cap);
+  return 0;
+}
+void spmv_decide(CsrDev &A, int maxrow, int cap)
+{
+  const int n = A.n;
   const double avg = n ? (double)A.nnz / n : 0.0;
   const char  *force = getenv("PERMON_B200_SPMV");   // "stream" | "vector" (A/B measurements)
   bool         stream = (cap <= 5632 && maxrow <= 64);   // <= 44 KB of products per tile
@@ -2009,7 +2030,6 @@ int spmv_config(CsrDev &A, const int *h_ia)
     else if (avg <= 24) W = 16;
     A.W = W;
   }
-  return 0;
 }
 
 // ---- epilogues ---------------------------------------------------------------------------------------

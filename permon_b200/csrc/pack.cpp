@@ -31,22 +31,8 @@
 
 namespace pb {
 
-static inline size_t up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+static inline size_t up(size_t v, size_t a) { return pk_up(v, a); }
 
-size_t pk_coded_bytes(int ndict, int nrows, int nnz, bool uniform)
-{
-  size_t b = sizeof(PkHeader) + up(ndict, 2) * 8 + up(ndict, 4) * 4;
-  if (!uniform) b += up((size_t)nrows + 1, 8) * 2;
-  b += up(nnz, 16);
-  return up(b, 16);
-}
-size_t pk_stencil_bytes(int L, int nrows) { return up(sizeof(PkHeader) + up(L, 2) * 8 + up(L, 4) * 4 + up((size_t)nrows, 16), 16); }
-size_t pk_raw_bytes(int nrows, int nnz)
-{
-  return up(sizeof(PkHeader) + up(nnz, 2) * 8 + up(nnz, 4) * 4 + up((size_t)nrows + 1, 8) * 2, 16);
-}
-
-namespace {
 // windows of a pattern: consecutive deltas within PB_ST_SPAN of the window's first delta share one; returns the last window index
 int pattern_windows(StPattern &P)
 {
@@ -64,6 +50,7 @@ int pattern_windows(StPattern &P)
   }
   return w;
 }
+namespace {
 struct TileDict {
   // open addressing over (delta, value bits); 1024 slots for at most 256 entries
   static constexpr int SLOTS = 1024;

@@ -1047,23 +1047,30 @@ static int upload_stencil(pb::CsrDev &C, pb::StencilHost &st, int64_t nnz, doubl
   C.st_masks = dm;
   C.st_pid   = dp;
   C.st_pats  = dt;
-  C.st_npat  = (int)st.pats.size();
-  C.st_nwin  = st.nwin;
-  C.st_lmax  = 0;
-  for (const pb::StPattern &P : st.pats) C.st_lmax = std::max(C.st_lmax, P.L);
+  stencil_set_fields(C, st.pats, st.nwin, st.masks.size(), st.pid.size());
+  return 0;
+}
+
+namespace pb {
+void stencil_set_fields(CsrDev &C, const std::vector<StPattern> &pats, int nwin, size_t masks_bytes, size_t npid)
+{
+  C.st_npat = (int)pats.size();
+  C.st_nwin = nwin;
+  C.st_lmax = 0;
+  for (const pb::StPattern &P : pats) C.st_lmax = std::max(C.st_lmax, P.L);
   C.st_dlo = C.st_dhi = 0;
-  for (const pb::StPattern &P : st.pats)
+  for (const pb::StPattern &P : pats)
     for (int j = 0; j < P.L; j++) {
       C.st_dlo = std::min(C.st_dlo, P.d[j]);
       C.st_dhi = std::max(C.st_dhi, P.d[j]);
     }
-  C.pk_bytes = (int64_t)st.masks.size() + (int64_t)st.pid.size() + (int64_t)(sizeof(pb::StPattern) * st.pats.size());
-  C.pk_coded = (int64_t)st.pid.size();
+  C.pk_bytes = (int64_t)masks_bytes + (int64_t)npid + (int64_t)(sizeof(pb::StPattern) * pats.size());
+  C.pk_coded = (int64_t)npid;
   C.kind     = 4;
   const char *stg = getenv("PERMON_B200_STAGES");
   C.stages = stg ? atoi(stg) : 0;   // 0: as many as fit
-  return 0;
 }
+}  // namespace pb
 
 static int upload_csr(pb::CsrDev &C, int nrows, int ncols, const int *ia, const int *ja, const double *a, const int *rows)
 {
@@ -1194,6 +1201,110 @@ PetscErrorCode MatCreateSeqAIJCUSPARSEWithArrays(MPI_Comm comm, PetscInt m, Pets
   return 0;
 }
 
+// whether a row-partitioned constructor first tries the all-stencil form of the diagonal block straight from the caller's arrays (one
+// pass, no copy of the block); shared by the host and the device constructor so that both build the same form
+static bool windowed_stencil_first(PetscInt m, PetscInt n)
+{
+  const char *e1 = getenv("PERMON_B200_ST_WINDOWS"), *e2 = getenv("PERMON_B200_PACK_STENCIL");
+  return m == n && m >= 64 && !getenv("PERMON_B200_EAGER_SPLIT") && !getenv("PERMON_B200_SPMV") && !(e1 && e1[0] == '0') && !(e2 && e2[0] == '0');
+}
+
+// the off-diagonal block from the ghost entries of a row block (row order, storage order within a row): ghost list (sorted unique global
+// columns), compressed rows with ghost-buffer columns, and the per-row "has ghosts" flags
+static void split_from_ghosts(const pb::OffDiagEntries &off, PetscInt m, std::vector<PetscInt> &gh, std::vector<int> &oia, std::vector<int> &oja,
+                            std::vector<double> &oa, std::vector<int> &orow, std::vector<unsigned char> &skip)
+{
+  skip.assign(std::max<PetscInt>(m, 1), 0);
+  gh.assign(off.gcol.begin(), off.gcol.end());
+  std::sort(gh.begin(), gh.end());
+  gh.erase(std::unique(gh.begin(), gh.end()), gh.end());
+  oja.resize(off.row.size());
+  oa.assign(off.val.begin(), off.val.end());
+  oia.assign(1, 0);
+  for (size_t k = 0; k < off.row.size(); k++) {
+    if (orow.empty() || orow.back() != off.row[k]) {
+      if (!orow.empty()) oia.push_back((int)k);
+      orow.push_back(off.row[k]);
+      skip[off.row[k]] = 1;
+    }
+    oja[k] = (int)(std::lower_bound(gh.begin(), gh.end(), (PetscInt)off.gcol[k]) - gh.begin());
+  }
+  if (!orow.empty()) oia.push_back((int)off.row.size());
+}
+
+// the rest of the halo plan once the ghost list (garray) and the off-diagonal rows are known: the widest ghost-free run of rows, the
+// neighbours that own the ghosts and, through the host exchange, the send lists (collective).  On a non-symmetric pattern the matrix is
+// destroyed on every rank and an error returned.
+static int halo_plan_finish(Mat A, const std::vector<int> &orow, const std::vector<int64_t> &cs)
+{
+  MPI_Comm                     comm = A->comm;
+  HaloPlan                    *H = A->halo;
+  const int                    size = comm->size, rank = comm->rank;
+  const PetscInt               m = A->m, c0 = A->cstart, c1 = A->cstart + A->n;
+  const std::vector<PetscInt> &gh = H->garray;
+  H->nboundary = (PetscInt)orow.size();
+  {   // widest run of interior rows: kernels skip the per-row flag lookup inside it
+    int best_lo = 0, best_hi = 0, cur = 0;
+    for (int r : orow) {
+      if (r - cur > best_hi - best_lo) best_lo = cur, best_hi = r;
+      cur = r + 1;
+    }
+    if ((int)m - cur > best_hi - best_lo) best_lo = cur, best_hi = (int)m;
+    H->skip_lo = best_lo;
+    H->skip_hi = best_hi;
+  }
+  // neighbours that own my ghosts
+  H->recv_off.push_back(0);
+  for (size_t g = 0; g < gh.size();) {
+    int owner = (int)(std::upper_bound(cs.begin(), cs.end(), (int64_t)gh[g]) - cs.begin()) - 1;
+    size_t e = g;
+    while (e < gh.size() && gh[e] < cs[owner + 1]) e++;
+    H->neigh.push_back(owner);
+    H->recv_off.push_back((PetscInt)e);
+    g = e;
+  }
+  // everybody publishes its ghost list; I pick what I own => my send lists (in the requester's ghost order)
+  std::vector<int64_t> gbytes(size);
+  if (comm->agi(comm->agctx, (int64_t)(gh.size() * sizeof(PetscInt)), gbytes.data())) return err(PETSC_ERR_LIB, "host all-gather failed");
+  int64_t tot = 0;
+  for (int r = 0; r < size; r++) tot += gbytes[r];
+  std::vector<PetscInt> allg((size_t)(tot / sizeof(PetscInt)) + 1);
+  if (comm->agv(comm->agctx, gh.data(), (int64_t)(gh.size() * sizeof(PetscInt)), allg.data(), gbytes.data())) return err(PETSC_ERR_LIB, "host all-gather failed");
+  {
+    std::vector<PetscInt> sneigh, soff(1, 0), sidx;
+    size_t                off = 0;
+    for (int r = 0; r < size; r++) {
+      size_t cnt = (size_t)(gbytes[r] / sizeof(PetscInt));
+      if (r != rank) {
+        size_t before = sidx.size();
+        for (size_t k = 0; k < cnt; k++) {
+          PetscInt g = allg[off + k];
+          if (g >= c0 && g < c1) sidx.push_back(g - c0);
+        }
+        if (sidx.size() > before) {
+          sneigh.push_back(r);
+          soff.push_back((PetscInt)sidx.size());
+        }
+      }
+      off += cnt;
+    }
+    // symmetric sparsity is assumed (Hessians are symmetric); every rank must take the same exit, or the others would hang in the next
+    // collective: agree on the flag first, then free the object through the normal destructor (halo plan and host split included)
+    std::vector<int64_t> oks(size);
+    if (comm->agi(comm->agctx, (int64_t)(sneigh == H->neigh), oks.data())) return err(PETSC_ERR_LIB, "host all-gather failed");
+    bool all_ok = true;
+    for (int r = 0; r < size; r++) all_ok = all_ok && oks[r];
+    if (!all_ok) {
+      Mat tmp = A;
+      MatDestroy(&tmp);
+      return err(PETSC_ERR_SUP, "non-symmetric halo pattern (send and receive neighbour sets differ on some rank)");
+    }
+    H->send_off = soff;
+    H->send_idx = sidx;
+  }
+  return 0;
+}
+
 // Row-partitioned AIJ: split into the diagonal block (local columns) and the off-diagonal block (ghost
 // columns, compressed rows), and build the halo plan -- the layout of PETSc's Mat_MPIAIJ
 // (include/permon/private/petsc/mpiaij.h:49-83: A, B, garray, lvec, Mvctx).
@@ -1257,8 +1368,7 @@ PetscErrorCode MatCreateMPIAIJWithArrays(MPI_Comm comm, PetscInt m, PetscInt n, 
   // all-stencil form -- one pass, no intermediate copy of the block; the ghost entries fall out of the same pass.
   bool fast = false;
   {
-    const char *e1 = getenv("PERMON_B200_ST_WINDOWS"), *e2 = getenv("PERMON_B200_PACK_STENCIL");
-    if (m == n && m >= 64 && !getenv("PERMON_B200_EAGER_SPLIT") && !getenv("PERMON_B200_SPMV") && !(e1 && e1[0] == '0') && !(e2 && e2[0] == '0')) {
+    if (windowed_stencil_first(m, n)) {
       pb::OffDiagEntries off;
       int64_t            nd = 0;
       PB_CHK(pb::pk_stencil_windowed((int)m, i, j, a, (int)c0, (int)n, H->host->st, off, nd));
@@ -1270,23 +1380,8 @@ PetscErrorCode MatCreateMPIAIJWithArrays(MPI_Comm comm, PetscInt m, PetscInt n, 
         H->host->uj = j;
         H->host->ua = a;
         H->host->c0 = c0;
-        skip.assign(std::max<PetscInt>(m, 1), 0);
-        gh.assign(off.gcol.begin(), off.gcol.end());
-        std::sort(gh.begin(), gh.end());
-        gh.erase(std::unique(gh.begin(), gh.end()), gh.end());
+        split_from_ghosts(off, m, gh, oia, oja, oa, orow, skip);
         H->garray = gh;
-        oja.resize(off.row.size());
-        oa.assign(off.val.begin(), off.val.end());
-        oia.assign(1, 0);
-        for (size_t k = 0; k < off.row.size(); k++) {
-          if (orow.empty() || orow.back() != off.row[k]) {
-            if (!orow.empty()) oia.push_back((int)k);
-            orow.push_back(off.row[k]);
-            skip[off.row[k]] = 1;
-          }
-          oja[k] = (int)(std::lower_bound(gh.begin(), gh.end(), (PetscInt)off.gcol[k]) - gh.begin());
-        }
-        if (!orow.empty()) oia.push_back((int)off.row.size());
       }
     }
   }
@@ -1352,67 +1447,8 @@ PetscErrorCode MatCreateMPIAIJWithArrays(MPI_Comm comm, PetscInt m, PetscInt n, 
     }
   }
   }
-  H->nboundary = (PetscInt)orow.size();
   const double t_s2 = wall_now();
-  {   // widest run of interior rows: kernels skip the per-row flag lookup inside it
-    int best_lo = 0, best_hi = 0, cur = 0;
-    for (int r : orow) {
-      if (r - cur > best_hi - best_lo) best_lo = cur, best_hi = r;
-      cur = r + 1;
-    }
-    if ((int)m - cur > best_hi - best_lo) best_lo = cur, best_hi = (int)m;
-    H->skip_lo = best_lo;
-    H->skip_hi = best_hi;
-  }
-  // neighbours that own my ghosts
-  H->recv_off.push_back(0);
-  for (size_t g = 0; g < gh.size();) {
-    int owner = (int)(std::upper_bound(cs.begin(), cs.end(), (int64_t)gh[g]) - cs.begin()) - 1;
-    size_t e = g;
-    while (e < gh.size() && gh[e] < cs[owner + 1]) e++;
-    H->neigh.push_back(owner);
-    H->recv_off.push_back((PetscInt)e);
-    g = e;
-  }
-  // everybody publishes its ghost list; I pick what I own => my send lists (in the requester's ghost order)
-  std::vector<int64_t> gbytes(size);
-  if (comm->agi(comm->agctx, (int64_t)(gh.size() * sizeof(PetscInt)), gbytes.data())) return err(PETSC_ERR_LIB, "host all-gather failed");
-  int64_t tot = 0;
-  for (int r = 0; r < size; r++) tot += gbytes[r];
-  std::vector<PetscInt> allg((size_t)(tot / sizeof(PetscInt)) + 1);
-  if (comm->agv(comm->agctx, gh.data(), (int64_t)(gh.size() * sizeof(PetscInt)), allg.data(), gbytes.data())) return err(PETSC_ERR_LIB, "host all-gather failed");
-  {
-    std::vector<PetscInt> sneigh, soff(1, 0), sidx;
-    size_t                off = 0;
-    for (int r = 0; r < size; r++) {
-      size_t cnt = (size_t)(gbytes[r] / sizeof(PetscInt));
-      if (r != rank) {
-        size_t before = sidx.size();
-        for (size_t k = 0; k < cnt; k++) {
-          PetscInt g = allg[off + k];
-          if (g >= c0 && g < c1) sidx.push_back(g - c0);
-        }
-        if (sidx.size() > before) {
-          sneigh.push_back(r);
-          soff.push_back((PetscInt)sidx.size());
-        }
-      }
-      off += cnt;
-    }
-    // symmetric sparsity is assumed (Hessians are symmetric); every rank must take the same exit, or the others would hang in the next
-    // collective: agree on the flag first, then free the object through the normal destructor (halo plan and host split included)
-    std::vector<int64_t> oks(size);
-    if (comm->agi(comm->agctx, (int64_t)(sneigh == H->neigh), oks.data())) return err(PETSC_ERR_LIB, "host all-gather failed");
-    bool all_ok = true;
-    for (int r = 0; r < size; r++) all_ok = all_ok && oks[r];
-    if (!all_ok) {
-      Mat tmp = A;
-      MatDestroy(&tmp);
-      return err(PETSC_ERR_SUP, "non-symmetric halo pattern (send and receive neighbour sets differ on some rank)");
-    }
-    H->send_off = soff;
-    H->send_idx = sidx;
-  }
+  PB_CHK(halo_plan_finish(A, orow, cs));
   if (verbose_timing())
     fprintf(stderr, "[permon_b200] rank %d host split of %d rows / %lld nnz: count + ghosts %.1f ms, fill %.1f ms, plan exchange %.1f ms\n", rank, (int)m,
             (long long)nnz, 1e3 * (t_s1 - t_s0), 1e3 * (t_s2 - t_s1), 1e3 * (wall_now() - t_s2));
@@ -1537,6 +1573,30 @@ static int halo_p2p_setup(Mat A)
   return 0;
 }
 
+// device side of the halo plan: send list, row map of the ghost rows, events (the off-diagonal rows `orow` of the split)
+static int halo_device_setup(Mat A, const std::vector<int> &orow)
+{
+  HaloPlan      *H = A->halo;
+  const PetscInt m = A->m;
+  PB_CHK(dmalloc(&H->d_send_idx, std::max<size_t>(H->send_idx.size(), 1)));
+  PB_CHK(dmalloc(&H->d_send, std::max<size_t>(H->send_idx.size(), 1)));
+  PB_CHK(dmalloc(&H->d_ghost, std::max<size_t>(H->garray.size(), 1)));
+  // rows outside the ghost-free run [skip_lo, skip_hi) -> their row in the compressed off-diagonal block (GhostMerge)
+  std::vector<int> row_map((size_t)std::max<PetscInt>(H->skip_lo + (m - H->skip_hi), 1), -1);
+  for (size_t q = 0; q < orow.size(); q++) {
+    const int r = orow[q];
+    row_map[r < H->skip_lo ? r : r - H->skip_hi + H->skip_lo] = (int)q;
+  }
+  PB_CHK(dmalloc(&H->d_row_map, row_map.size()));
+  PB_CUDA(cudaMemcpyAsync(H->d_send_idx, H->send_idx.data(), sizeof(int) * H->send_idx.size(), cudaMemcpyHostToDevice, ctx().stream));
+  PB_CUDA(cudaMemcpyAsync(H->d_row_map, row_map.data(), sizeof(int) * row_map.size(), cudaMemcpyHostToDevice, ctx().stream));
+  PB_CUDA(cudaEventCreateWithFlags(&H->ev_packed, cudaEventDisableTiming));
+  PB_CUDA(cudaEventCreateWithFlags(&H->ev_arrived, cudaEventDisableTiming));
+  PB_CUDA(cudaEventCreateWithFlags(&H->ev_consumed, cudaEventDisableTiming));
+  PB_CUDA(cudaStreamSynchronize(ctx().stream));
+  return 0;
+}
+
 namespace pb {
 int mat_ensure_device(Mat A)
 {
@@ -1560,22 +1620,7 @@ int mat_ensure_device(Mat A)
     PB_CHK(upload_csr(A->Ad, m, A->n, S->dia.data(), S->dja.data(), S->da.data(), nullptr));
   }
   PB_CHK(upload_csr(A->Ao, (int)S->orow.size(), (int)H->garray.size(), S->oia.data(), S->oja.data(), S->oa.data(), S->orow.data()));
-  PB_CHK(dmalloc(&H->d_send_idx, std::max<size_t>(H->send_idx.size(), 1)));
-  PB_CHK(dmalloc(&H->d_send, std::max<size_t>(H->send_idx.size(), 1)));
-  PB_CHK(dmalloc(&H->d_ghost, std::max<size_t>(H->garray.size(), 1)));
-  // rows outside the ghost-free run [skip_lo, skip_hi) -> their row in the compressed off-diagonal block (GhostMerge)
-  std::vector<int> row_map((size_t)std::max<PetscInt>(H->skip_lo + (m - H->skip_hi), 1), -1);
-  for (size_t q = 0; q < S->orow.size(); q++) {
-    const int r = S->orow[q];
-    row_map[r < H->skip_lo ? r : r - H->skip_hi + H->skip_lo] = (int)q;
-  }
-  PB_CHK(dmalloc(&H->d_row_map, row_map.size()));
-  PB_CUDA(cudaMemcpyAsync(H->d_send_idx, H->send_idx.data(), sizeof(int) * H->send_idx.size(), cudaMemcpyHostToDevice, ctx().stream));
-  PB_CUDA(cudaMemcpyAsync(H->d_row_map, row_map.data(), sizeof(int) * row_map.size(), cudaMemcpyHostToDevice, ctx().stream));
-  PB_CUDA(cudaEventCreateWithFlags(&H->ev_packed, cudaEventDisableTiming));
-  PB_CUDA(cudaEventCreateWithFlags(&H->ev_arrived, cudaEventDisableTiming));
-  PB_CUDA(cudaEventCreateWithFlags(&H->ev_consumed, cudaEventDisableTiming));
-  PB_CUDA(cudaStreamSynchronize(ctx().stream));
+  PB_CHK(halo_device_setup(A, S->orow));
   delete S;
   H->host = nullptr;
   if (A->comm->p2p) PB_CHK(halo_p2p_setup(A));
@@ -1642,6 +1687,200 @@ PetscErrorCode MatB200GetStorageInfo(Mat A, PetscInt *kind, PetscReal *stream_by
   if (stream_bytes) *stream_bytes = pb::csr_stream_bytes(A->Ad) + (A->halo ? pb::csr_stream_bytes(A->Ao) : 0.0);
   if (coded_tiles) *coded_tiles = (PetscInt)A->Ad.pk_coded;
   if (tiles) *tiles = (A->Ad.n + pb::TR - 1) / pb::TR;
+  return 0;
+}
+
+static int check_device_array(const void *p, const char *what)
+{
+  cudaPointerAttributes at;
+  if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+    cudaGetLastError();
+    return err(PETSC_ERR_ARG_WRONG, "%s: not a CUDA pointer", what);
+  }
+  if (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) return err(PETSC_ERR_ARG_WRONG, "%s: host memory, a device pointer is required", what);
+  if (at.device != ctx().device) return err(PETSC_ERR_ARG_WRONG, "%s: memory of device %d, the library runs on device %d", what, at.device, ctx().device);
+  return 0;
+}
+
+// Row-partitioned (or one-rank) AIJ from a CSR in device memory, re-coded on the device into the form upload_csr builds from a host CSR
+// (recode.cu).  On several ranks the split into the diagonal and off-diagonal block runs on the device too; only the ghost entries reach
+// the host, where the halo plan is built exactly as for MatCreateMPIAIJWithArrays.  Nothing of the caller's arrays is kept.
+PetscErrorCode MatB200CreateAIJWithDeviceArrays(MPI_Comm comm, PetscInt m, PetscInt n, PetscInt M, PetscInt N, const PetscInt di[], const PetscInt dj[],
+                                                const PetscScalar da[], Mat *mat)
+{
+  (void)M;
+  (void)N;
+  if (!mat) return err(PETSC_ERR_ARG_NULL, "null Mat pointer");
+  if (n == PETSC_DECIDE) n = m;
+  if (!di) return err(PETSC_ERR_ARG_NULL, "null row pointer");
+  PB_CHK(dev_init());
+  PB_CHK(check_device_array(di, "row pointer"));
+  cudaStream_t s   = ctx().stream;
+  int          nnz = 0;
+  PB_CUDA(cudaMemcpyAsync(&nnz, di + m, sizeof(int), cudaMemcpyDeviceToHost, s));
+  PB_CUDA(cudaStreamSynchronize(s));
+  if (nnz > 0) {
+    if (!dj || !da) return err(PETSC_ERR_ARG_NULL, "null CSR array");
+    PB_CHK(check_device_array(dj, "column ids"));
+    PB_CHK(check_device_array(da, "values"));
+  }
+  PhaseTimer pt("MatB200CreateAIJWithDeviceArrays");
+  if (comm->size == 1) {
+    _p_Mat *A = new _p_Mat;
+    A->comm   = comm;
+    A->kind   = MK_AIJ;
+    A->m = A->M = m;
+    A->n = A->N = n;
+    int ierr = pb::recode_csr_dev(A->Ad, m, n, di, dj, da);
+    if (!ierr) ierr = cudaStreamSynchronize(s) == cudaSuccess ? 0 : err(PETSC_ERR_GPU, "%s", cudaGetErrorString(cudaGetLastError()));
+    if (ierr) {
+      delete A;
+      return ierr;
+    }
+    *mat = A;
+    return 0;
+  }
+  if (!comm->agi || !comm->agv) return err(PETSC_ERR_ARG_WRONGSTATE, "communicator has no host exchange");
+  const int            size = comm->size, rank = comm->rank;
+  std::vector<int64_t> rows_all(size), cols_all(size);
+  if (comm->agi(comm->agctx, m, rows_all.data()) || comm->agi(comm->agctx, n, cols_all.data())) return err(PETSC_ERR_LIB, "host all-gather failed");
+  std::vector<int64_t> rs(size + 1, 0), cs(size + 1, 0);
+  for (int r = 0; r < size; r++) {
+    rs[r + 1] = rs[r] + rows_all[r];
+    cs[r + 1] = cs[r] + cols_all[r];
+  }
+  _p_Mat *A = new _p_Mat;
+  A->comm   = comm;
+  A->kind   = MK_AIJ;
+  A->m      = m;
+  A->n      = n;
+  A->M      = (PetscInt)rs[size];
+  A->N      = (PetscInt)cs[size];
+  A->rstart = (PetscInt)rs[rank];
+  A->cstart = (PetscInt)cs[rank];
+  if (A->M <= PB_MAXEQ_ALL && A->M != A->N) {
+    // equality rows (at most PB_MAXEQ_ALL in all): kept on the host like MatCreateMPIAIJWithArrays keeps them
+    A->eq_host = new _p_Mat::EqHost;
+    A->eq_host->ia.resize((size_t)m + 1);
+    A->eq_host->ja.resize((size_t)nnz);
+    A->eq_host->a.resize((size_t)nnz);
+    PB_CUDA(cudaMemcpyAsync(A->eq_host->ia.data(), di, sizeof(int) * ((size_t)m + 1), cudaMemcpyDeviceToHost, s));
+    PB_CUDA(cudaMemcpyAsync(A->eq_host->ja.data(), dj, sizeof(int) * (size_t)nnz, cudaMemcpyDeviceToHost, s));
+    PB_CUDA(cudaMemcpyAsync(A->eq_host->a.data(), da, sizeof(double) * (size_t)nnz, cudaMemcpyDeviceToHost, s));
+    PB_CUDA(cudaStreamSynchronize(s));
+    A->Ad.n     = m;
+    A->Ad.ncols = n;
+    A->Ad.nnz   = nnz;
+    *mat        = A;
+    return 0;
+  }
+  HaloPlan *H = new HaloPlan;
+  A->halo     = H;
+  auto fail = [&](int ierr) {
+    Mat tmp = A;
+    MatDestroy(&tmp);
+    return ierr;
+  };
+  // the diagonal block: all-stencil straight from the caller's arrays when the host constructor would try that too (same rule), else
+  // a device split into a library-owned CSR with local columns that goes through the general re-coder (and is adopted if it stays CSR)
+  bool st_done = false;
+  int  ierr    = 0;
+  if (windowed_stencil_first(m, n)) ierr = pb::recode_stencil_window_dev(A->Ad, (int)m, di, dj, da, (int)A->cstart, (int)n, &st_done);
+  int               *sia = nullptr, *sja = nullptr;
+  double            *sa  = nullptr;
+  pb::OffDiagEntries off;
+  if (!ierr) ierr = pb::split_rows_dev((int)m, di, dj, da, (int)A->cstart, (int)n, !st_done, &sia, &sja, &sa, off);
+  if (!ierr && !st_done) ierr = pb::recode_csr_dev(A->Ad, m, n, sia, sja, sa, &sia, &sja, &sa);
+  dfree(sia);
+  dfree(sja);
+  dfree(sa);
+  if (ierr) return fail(ierr);
+  std::vector<int>           oia, oja, orow;
+  std::vector<double>        oa;
+  std::vector<unsigned char> skip;
+  std::vector<PetscInt>      gh;
+  split_from_ghosts(off, m, gh, oia, oja, oa, orow, skip);
+  H->garray = gh;
+  PB_CHK(halo_plan_finish(A, orow, cs));   // destroys A itself on a non-symmetric pattern
+  ierr = upload_csr(A->Ao, (int)orow.size(), (int)H->garray.size(), oia.data(), oja.data(), oa.data(), orow.data());
+  if (!ierr) ierr = halo_device_setup(A, orow);
+  if (!ierr && comm->p2p) ierr = halo_p2p_setup(A);
+  if (!ierr && cudaStreamSynchronize(s) != cudaSuccess) ierr = err(PETSC_ERR_GPU, "%s", cudaGetErrorString(cudaGetLastError()));
+  if (ierr) return fail(ierr);
+  *mat = A;
+  return 0;
+}
+
+PetscErrorCode MatB200GetStoredForm(Mat A, PetscInt part, void *buf, size_t *nbytes)
+{
+  if (!A || A->kind != MK_AIJ) return err(PETSC_ERR_ARG_WRONG, "MatB200GetStoredForm: AIJ matrix expected");
+  if (!nbytes) return err(PETSC_ERR_ARG_NULL, "null size pointer");
+  const int block = (int)(part / MATB200_FORM_OFFDIAG), field = (int)(part % MATB200_FORM_OFFDIAG);
+  if (part < 0 || block > 1) return err(PETSC_ERR_ARG_OUTOFRANGE, "MatB200GetStoredForm: unknown part %d", (int)part);
+  if (!A->eq_host) PB_CHK(pb::mat_ensure_device(A));
+  static const pb::CsrDev none;
+  const pb::CsrDev       &C = block == 0 ? A->Ad : (A->halo ? A->Ao : none);
+  const size_t            ntiles = (size_t)(C.n + pb::TR - 1) / pb::TR;
+  const void             *src = nullptr;
+  bool                    host = false;
+  size_t                  sz = 0;
+  int64_t                 sc[15];
+  switch (field) {
+  case MATB200_FORM_SCALARS: {
+    const int64_t v[15] = {C.kind, C.n, C.ncols, C.nnz, C.st_npat, C.st_nwin, C.st_lmax, C.st_dlo, C.st_dhi, C.pk_max, C.pk_bytes, C.pk_coded, C.stages, C.tile_cap, C.W};
+    memcpy(sc, v, sizeof sc);
+    src  = sc;
+    host = true;
+    sz   = sizeof sc;
+    break;
+  }
+  case MATB200_FORM_ST_MASKS: src = C.st_masks, sz = C.st_masks ? ntiles * pb::TR : 0; break;
+  case MATB200_FORM_ST_PID: src = C.st_pid, sz = C.st_pid ? ntiles : 0; break;
+  case MATB200_FORM_ST_PATS: src = C.st_pats, sz = C.st_pats ? sizeof(pb::StPattern) * (size_t)C.st_npat : 0; break;
+  case MATB200_FORM_PK_BLOB:
+    src = C.pk;
+    if (C.pk) {
+      unsigned last = 0;
+      PB_CUDA(cudaMemcpy(&last, C.pk_off + ntiles, sizeof last, cudaMemcpyDeviceToHost));
+      sz = (size_t)last * 16 + 16;
+    }
+    break;
+  case MATB200_FORM_PK_OFF: src = C.pk_off, sz = C.pk_off ? sizeof(unsigned) * (ntiles + 1) : 0; break;
+  case MATB200_FORM_CSR_IA:
+  case MATB200_FORM_CSR_JA:
+  case MATB200_FORM_CSR_A:
+    if (block == 0 && A->eq_host) {
+      host = true;
+      if (field == MATB200_FORM_CSR_IA) src = A->eq_host->ia.data(), sz = sizeof(int) * A->eq_host->ia.size();
+      if (field == MATB200_FORM_CSR_JA) src = A->eq_host->ja.data(), sz = sizeof(int) * A->eq_host->ja.size();
+      if (field == MATB200_FORM_CSR_A) src = A->eq_host->a.data(), sz = sizeof(double) * A->eq_host->a.size();
+    } else {
+      if (field == MATB200_FORM_CSR_IA) src = C.ia, sz = C.ia ? sizeof(int) * ((size_t)C.n + 1) : 0;
+      if (field == MATB200_FORM_CSR_JA) src = C.ja, sz = C.ja ? sizeof(int) * (size_t)C.nnz : 0;
+      if (field == MATB200_FORM_CSR_A) src = C.a, sz = C.a ? sizeof(double) * (size_t)C.nnz : 0;
+    }
+    break;
+  case MATB200_FORM_ELL_VAL: src = C.ell_val, sz = C.ell_val ? sizeof(double) * (size_t)C.ell_elems : 0; break;
+  case MATB200_FORM_ELL_COL: src = C.ell_col, sz = C.ell_col ? sizeof(int) * (size_t)C.ell_elems : 0; break;
+  case MATB200_FORM_ELL_LEN: src = C.ell_len, sz = C.ell_len ? sizeof(int) * (size_t)C.n : 0; break;
+  case MATB200_FORM_ELL_LT: src = C.ell_lt, sz = C.ell_lt ? sizeof(int) * ntiles : 0; break;
+  case MATB200_FORM_ELL_OFF: src = C.ell_off, sz = C.ell_off ? sizeof(int64_t) * ntiles : 0; break;
+  case MATB200_FORM_ROWS: src = C.rows, sz = C.rows ? sizeof(int) * (size_t)C.n : 0; break;
+  default: return err(PETSC_ERR_ARG_OUTOFRANGE, "MatB200GetStoredForm: unknown part %d", (int)part);
+  }
+  if (!buf) {
+    *nbytes = sz;
+    return 0;
+  }
+  if (*nbytes < sz) return err(PETSC_ERR_ARG_SIZ, "MatB200GetStoredForm: buffer of %zu bytes, %zu needed", *nbytes, sz);
+  if (sz) {
+    if (host) memcpy(buf, src, sz);
+    else {
+      PB_CUDA(cudaStreamSynchronize(ctx().stream));
+      PB_CUDA(cudaMemcpy(buf, src, sz, cudaMemcpyDeviceToHost));
+    }
+  }
+  *nbytes = sz;
   return 0;
 }
 
