@@ -93,6 +93,23 @@ PetscErrorCode MatCreateOneRow(Vec a, Mat *A)
   (*A)->m = 1; (*A)->n = a->n; (*A)->row = a;
   return 0;
 }
+PetscErrorCode MatCreateSeqDense(MPI_Comm comm, PetscInt m, PetscInt n, PetscScalar *data, Mat *A)
+{   /* column-major, entry (i, j) at data[i + j * lda], lda = m until MatDenseSetLDA (the user's array; no allocation by the mock) */
+  PetscCall(PetscNew(A));
+  (*A)->hdr.type_name = MATSEQDENSE;
+  (*A)->hdr.comm      = comm;
+  (*A)->m = m; (*A)->n = n; (*A)->a = data; (*A)->lda = m > 0 ? m : 1;
+  return 0;
+}
+PetscErrorCode MatDenseSetLDA(Mat A, PetscInt lda)
+{
+  PetscCheck(lda >= A->m, PETSC_COMM_SELF, PETSC_ERR_SUP, "lda %d < %d rows", (int)lda, (int)A->m);
+  A->lda = lda;
+  return 0;
+}
+PetscErrorCode MatDenseGetLDA(Mat A, PetscInt *lda) { *lda = A->lda; return 0; }
+PetscErrorCode MatDenseGetArrayRead(Mat A, const PetscScalar **a) { *a = A->a; return 0; }
+PetscErrorCode MatDenseRestoreArrayRead(Mat A, const PetscScalar **a) { (void)A; *a = NULL; return 0; }
 PetscErrorCode MatDestroy(Mat *A) { free(*A); *A = NULL; return 0; }
 PetscErrorCode MatGetSize(Mat A, PetscInt *M, PetscInt *N) { *M = A->m; *N = A->n; return 0; }
 PetscErrorCode MatGetLocalSize(Mat A, PetscInt *m, PetscInt *n) { *m = A->m; *n = A->n; return 0; }

@@ -1,7 +1,7 @@
 /* permon_mock.h -- TEST INFRASTRUCTURE: the smallest stand-in for the PETSc / PERMON headers that adapters/qpsb200.c touches, so that the
  * adapter compiles and RUNS in this repository, where PETSc does not exist.  Shapes follow the reference (include/permon/private/
  * qpsimpl.h:12-71 for _QPSOps / _p_QPS; petscsys.h conventions for PetscCall / PetscCheck / PetscObject).  Sequential only (one rank);
- * Mat = host CSR, Vec = host array.  Not part of the product: libpermon_b200.so never sees this file. */
+ * Mat = host CSR or a column-major dense array (MATSEQDENSE), Vec = host array.  Not part of the product: libpermon_b200.so never sees this file. */
 #ifndef PERMON_MOCK_H
 #define PERMON_MOCK_H
 #include <stdio.h>
@@ -35,6 +35,7 @@ typedef enum { MAT_INITIAL_MATRIX, MAT_REUSE_MATRIX } MatReuse;
 #define PetscInt_FMT "d"
 #define PERMON_EXTERN extern
 #define MATSEQAIJ "seqaij"
+#define MATSEQDENSE "seqdense"
 #define MATONEROW "onerow"
 #define QPCBOX "box"
 #define QPSMPGP "mpgp"
@@ -85,7 +86,7 @@ typedef struct _p_QPS *QPS;
 typedef struct _p_PetscViewer *PetscViewer;
 struct _p_PetscViewer { struct _p_PetscObject hdr; FILE *f; };
 struct _p_Vec { struct _p_PetscObject hdr; PetscInt n; PetscScalar *a; PetscBool owned; };
-struct _p_Mat { struct _p_PetscObject hdr; PetscInt m, n; PetscInt *ia, *ja; PetscScalar *a; Vec row; /* MATONEROW */ };
+struct _p_Mat { struct _p_PetscObject hdr; PetscInt m, n; PetscInt *ia, *ja; PetscScalar *a; Vec row; /* MATONEROW */ PetscInt lda; /* MATSEQDENSE */ };
 struct _p_QPC { struct _p_PetscObject hdr; Vec lb, ub; };
 struct _p_QP  { struct _p_PetscObject hdr; Mat A, BE; Vec b, x, cE; QPC qpc; };
 
@@ -128,6 +129,11 @@ PetscErrorCode PetscViewerASCIIPrintf(PetscViewer v, const char *fmt, ...);
 
 PetscErrorCode MatCreateSeqAIJWithArrays(MPI_Comm comm, PetscInt m, PetscInt n, PetscInt *i, PetscInt *j, PetscScalar *a, Mat *A);
 PetscErrorCode MatCreateOneRow(Vec a, Mat *A);
+PetscErrorCode MatCreateSeqDense(MPI_Comm comm, PetscInt m, PetscInt n, PetscScalar *data, Mat *A);
+PetscErrorCode MatDenseSetLDA(Mat A, PetscInt lda);
+PetscErrorCode MatDenseGetLDA(Mat A, PetscInt *lda);
+PetscErrorCode MatDenseGetArrayRead(Mat A, const PetscScalar **a);
+PetscErrorCode MatDenseRestoreArrayRead(Mat A, const PetscScalar **a);
 PetscErrorCode MatDestroy(Mat *A);
 PetscErrorCode MatGetSize(Mat A, PetscInt *M, PetscInt *N);
 PetscErrorCode MatGetLocalSize(Mat A, PetscInt *m, PetscInt *n);

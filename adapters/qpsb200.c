@@ -9,6 +9,7 @@
  *   struct _QPSOps, struct _p_QPS          include/permon/private/qpsimpl.h:12-71   (every slot of the vtable is filled below)
  *   QPSCreate_MPGP / QPSCreate_SMALXE      src/qps/impls/mpgp/mpgp.c:819-869, src/qps/impls/smalxe/smalxe.c:1143-1207
  *   Mat_MPIAIJ row-partitioned layout      include/permon/private/petsc/mpiaij.h:49-83 (read through MatMPIAIJGetLocalMat)
+ *   MATSEQDENSE Hessians                   column-major host array + leading dimension (MatDenseGetArrayRead, MatDenseGetLDA)
  *
  * The adapter is thin on purpose: it reads the PETSc objects of the QP (host CSR of the local rows with GLOBAL column indices, host
  * arrays of the vectors), hands them to the C ABI of libpermon_b200.so (include/permon_b200.h) -- "uploaded once" -- and lets the whole
@@ -45,6 +46,8 @@ typedef struct {
   int (*PetscOptionsInsertString)(void *, const char *);
   int (*MatCreateMPIAIJWithArrays)(void *, b200_int, b200_int, b200_int, b200_int, const b200_int *, const b200_int *, const double *, void **);
   int (*MatCreateOneRow)(void *, void **);
+  int (*MatCreateSeqDense)(void *, b200_int, b200_int, double *, void **);
+  int (*MatDenseSetLDA)(void *, b200_int);
   int (*MatDestroy)(void **);
   int (*VecCreateMPIWithArray)(void *, b200_int, b200_int, b200_int, const double *, void **);
   int (*VecGetArrayRead)(void *, const double **);
@@ -105,7 +108,7 @@ static PetscErrorCode B200Load(void)
   PetscCheck(g_b200.comm_world, PETSC_COMM_SELF, PETSC_ERR_LIB, "libpermon_b200.so does not export PETSC_COMM_WORLD");
   B200_BIND(PermonInitialize); B200_BIND(PermonB200GetUniqueId); B200_BIND(PermonB200CommInitRank); B200_BIND(PermonB200GetLastErrorMessage);
   B200_BIND(PetscOptionsInsertString);
-  B200_BIND(MatCreateMPIAIJWithArrays); B200_BIND(MatCreateOneRow); B200_BIND(MatDestroy);
+  B200_BIND(MatCreateMPIAIJWithArrays); B200_BIND(MatCreateOneRow); B200_BIND(MatCreateSeqDense); B200_BIND(MatDenseSetLDA); B200_BIND(MatDestroy);
   B200_BIND(VecCreateMPIWithArray); B200_BIND(VecGetArrayRead); B200_BIND(VecRestoreArrayRead); B200_BIND(VecDestroy);
   B200_BIND(QPCreate); B200_BIND(QPDestroy); B200_BIND(QPSetOperator); B200_BIND(QPSetRhs); B200_BIND(QPSetInitialVector); B200_BIND(QPSetBox); B200_BIND(QPSetEq);
   B200_BIND(QPSCreate); B200_BIND(QPSDestroy); B200_BIND(QPSSetType); B200_BIND(QPSSetQP); B200_BIND(QPSSetTolerances); B200_BIND(QPSSetOptionsPrefix);
@@ -146,6 +149,8 @@ typedef struct {
   PetscBool          Aloc_owned;
   const PetscInt    *ia, *ja;
   const PetscScalar *a, *pb, *plb, *pub, *pbe, *pce;
+  const PetscScalar *ad; /* MATSEQDENSE Hessian: its column-major array (of Adense), borrowed until the next set-up / reset */
+  Mat                Adense;
   PetscScalar       *px;
   Vec                vb, vx, vlb, vub, vbe, vce;
   PetscInt           nrows;
@@ -167,6 +172,7 @@ static PetscErrorCode B200ReleaseBorrowed(QPS_B200 *ctx)
   }
   if (ctx->pce) PetscCall(VecRestoreArrayRead(ctx->vce, &ctx->pce));
   if (ctx->a) PetscCall(MatSeqAIJRestoreArrayRead(ctx->Aloc, &ctx->a));
+  if (ctx->ad) PetscCall(MatDenseRestoreArrayRead(ctx->Adense, &ctx->ad));
   if (ctx->ia) PetscCall(MatRestoreRowIJ(ctx->Aloc, 0, PETSC_FALSE, PETSC_FALSE, &ctx->nrows, &ctx->ia, &ctx->ja, &done));
   if (ctx->Aloc_owned) PetscCall(MatDestroy(&ctx->Aloc));
   free(ctx->ia32);
@@ -174,6 +180,8 @@ static PetscErrorCode B200ReleaseBorrowed(QPS_B200 *ctx)
   ctx->pb = ctx->plb = ctx->pub = ctx->pbe = ctx->pce = NULL;
   ctx->px = NULL;
   ctx->a  = NULL;
+  ctx->ad = NULL;
+  ctx->Adense = NULL;
   ctx->ia = ctx->ja = NULL;
   ctx->ia32 = ctx->ja32 = NULL;
   ctx->Aloc             = NULL;
@@ -206,7 +214,7 @@ static PetscErrorCode QPSSetUp_B200(QPS qps)
   Vec         b, x, lb = NULL, ub = NULL, cE = NULL;
   IS          is = NULL;
   PetscInt    m, n, M, N;
-  PetscBool   done, isseq;
+  PetscBool   done, isseq, isdense;
   void       *comm;
   const char *prefix = NULL;
 
@@ -222,34 +230,46 @@ static PetscErrorCode QPSSetUp_B200(QPS qps)
   PetscCall(QPGetEq(qp, &BE, &cE));
   PetscCheck(!is, PetscObjectComm((PetscObject)qps), PETSC_ERR_SUP, "box constraints on an index subset: expand lb / ub to full length (-infinity / +infinity) first");
 
-  /* Hessian: local rows, GLOBAL column indices (what MatCreateMPIAIJWithArrays of either side takes).  MPIAIJ keeps a diagonal and an
-     off-diagonal block with compressed local columns (mpiaij.h:49-83); MatMPIAIJGetLocalMat merges them back */
   PetscCall(MatGetSize(A, &M, &N));
   PetscCall(MatGetLocalSize(A, &m, &n));
-  PetscCall(PetscObjectTypeCompare((PetscObject)A, MATSEQAIJ, &isseq));
-  if (isseq) {
-    ctx->Aloc       = A;
-    ctx->Aloc_owned = PETSC_FALSE;
+  PetscCall(PetscObjectTypeCompare((PetscObject)A, MATSEQDENSE, &isdense));
+  if (isdense) {
+    /* dense Hessian (one rank): PETSc's column-major array (entry (i, j) at a[i + j*lda]) and its leading dimension go over as they are.
+       The library copies the array to the device at the first use (QPSSetUp below); it stays borrowed until the next set-up or reset */
+    PetscInt lda;
+    PetscCall(MatDenseGetLDA(A, &lda));
+    PetscCall(MatDenseGetArrayRead(A, &ctx->ad));
+    ctx->Adense = A;
+    B200_CALL(g_b200.MatCreateSeqDense(comm, (b200_int)M, (b200_int)N, (double *)ctx->ad, &ctx->A));
+    if (lda != M) B200_CALL(g_b200.MatDenseSetLDA(ctx->A, (b200_int)lda));
   } else {
-    PetscCall(MatMPIAIJGetLocalMat(A, MAT_INITIAL_MATRIX, &ctx->Aloc));
-    ctx->Aloc_owned = PETSC_TRUE;
-  }
-  PetscCall(MatGetRowIJ(ctx->Aloc, 0, PETSC_FALSE, PETSC_FALSE, &ctx->nrows, &ctx->ia, &ctx->ja, &done));
-  PetscCheck(done && ctx->nrows == m, PetscObjectComm((PetscObject)qps), PETSC_ERR_SUP, "the Hessian must be an assembled (MPI)AIJ matrix");
-  PetscCall(MatSeqAIJGetArrayRead(ctx->Aloc, &ctx->a));
-  {
-    const b200_int *ia = (const b200_int *)ctx->ia, *ja = (const b200_int *)ctx->ja;
-    if (sizeof(PetscInt) != sizeof(b200_int)) { /* 64-bit-index PETSc: the device CSR is int32 */
-      PetscInt k, nz = ctx->ia[m];
-      PetscCheck(M < 2147483647 && nz < 2147483647, PetscObjectComm((PetscObject)qps), PETSC_ERR_SUP, "local block too large for 32-bit indices");
-      ctx->ia32 = (b200_int *)malloc(sizeof(b200_int) * (size_t)(m + 1));
-      ctx->ja32 = (b200_int *)malloc(sizeof(b200_int) * (size_t)(nz > 0 ? nz : 1));
-      for (k = 0; k <= m; k++) ctx->ia32[k] = (b200_int)ctx->ia[k];
-      for (k = 0; k < nz; k++) ctx->ja32[k] = (b200_int)ctx->ja[k];
-      ia = ctx->ia32;
-      ja = ctx->ja32;
+    /* AIJ Hessian: local rows, GLOBAL column indices (what MatCreateMPIAIJWithArrays of either side takes).  MPIAIJ keeps a diagonal and
+       an off-diagonal block with compressed local columns (mpiaij.h:49-83); MatMPIAIJGetLocalMat merges them back */
+    PetscCall(PetscObjectTypeCompare((PetscObject)A, MATSEQAIJ, &isseq));
+    if (isseq) {
+      ctx->Aloc       = A;
+      ctx->Aloc_owned = PETSC_FALSE;
+    } else {
+      PetscCall(MatMPIAIJGetLocalMat(A, MAT_INITIAL_MATRIX, &ctx->Aloc));
+      ctx->Aloc_owned = PETSC_TRUE;
     }
-    B200_CALL(g_b200.MatCreateMPIAIJWithArrays(comm, (b200_int)m, (b200_int)n, (b200_int)M, (b200_int)N, ia, ja, ctx->a, &ctx->A));
+    PetscCall(MatGetRowIJ(ctx->Aloc, 0, PETSC_FALSE, PETSC_FALSE, &ctx->nrows, &ctx->ia, &ctx->ja, &done));
+    PetscCheck(done && ctx->nrows == m, PetscObjectComm((PetscObject)qps), PETSC_ERR_SUP, "the Hessian must be an assembled (MPI)AIJ matrix");
+    PetscCall(MatSeqAIJGetArrayRead(ctx->Aloc, &ctx->a));
+    {
+      const b200_int *ia = (const b200_int *)ctx->ia, *ja = (const b200_int *)ctx->ja;
+      if (sizeof(PetscInt) != sizeof(b200_int)) { /* 64-bit-index PETSc: the device CSR is int32 */
+        PetscInt k, nz = ctx->ia[m];
+        PetscCheck(M < 2147483647 && nz < 2147483647, PetscObjectComm((PetscObject)qps), PETSC_ERR_SUP, "local block too large for 32-bit indices");
+        ctx->ia32 = (b200_int *)malloc(sizeof(b200_int) * (size_t)(m + 1));
+        ctx->ja32 = (b200_int *)malloc(sizeof(b200_int) * (size_t)(nz > 0 ? nz : 1));
+        for (k = 0; k <= m; k++) ctx->ia32[k] = (b200_int)ctx->ia[k];
+        for (k = 0; k < nz; k++) ctx->ja32[k] = (b200_int)ctx->ja[k];
+        ia = ctx->ia32;
+        ja = ctx->ja32;
+      }
+      B200_CALL(g_b200.MatCreateMPIAIJWithArrays(comm, (b200_int)m, (b200_int)n, (b200_int)M, (b200_int)N, ia, ja, ctx->a, &ctx->A));
+    }
   }
 
   /* vectors: the library adopts the host arrays; x stays the solution storage */

@@ -189,6 +189,24 @@ PERMON_EXTERN PetscErrorCode MatCreateSeqAIJWithArrays(MPI_Comm comm, PetscInt m
 PERMON_EXTERN PetscErrorCode MatCreateMPIAIJWithArrays(MPI_Comm comm, PetscInt m, PetscInt n, PetscInt M, PetscInt N, const PetscInt i[], const PetscInt j[], const PetscScalar a[], Mat *mat);
 /* same, from CUDA device pointers (int32 rowptr/cols, fp64 values): nothing crosses PCIe */
 PERMON_EXTERN PetscErrorCode MatCreateSeqAIJCUSPARSEWithArrays(MPI_Comm comm, PetscInt m, PetscInt n, const PetscInt di[], const PetscInt dj[], const PetscScalar da[], Mat *mat);
+/* Dense matrices, column-major as MATSEQDENSE: entry (i, j) at data[i + j * lda], lda = m unless MatDenseSetLDA says otherwise (before the
+   first use).  One rank only.  A host array is copied to the device at the first use (MatMult, a solver set-up, MatB200GetDenseInfo): it
+   must stay valid until then, later writes to it are not seen.  A device array (MatCreateSeqDenseCUDA) is read in place on every product
+   when its base is 16-byte aligned and lda is even; otherwise the first use makes one padded device copy.  Freeing it is the caller's
+   business, after the matrix is destroyed. */
+/* petscmat.h: PetscErrorCode MatCreateSeqDense(MPI_Comm, PetscInt, PetscInt, PetscScalar[], Mat *) */
+PERMON_EXTERN PetscErrorCode MatCreateSeqDense(MPI_Comm comm, PetscInt m, PetscInt n, PetscScalar data[], Mat *A);
+/* petscmat.h: PetscErrorCode MatCreateSeqDenseCUDA(MPI_Comm, PetscInt, PetscInt, PetscScalar[], Mat *) */
+PERMON_EXTERN PetscErrorCode MatCreateSeqDenseCUDA(MPI_Comm comm, PetscInt m, PetscInt n, PetscScalar data[], Mat *A);
+/* petscmat.h: PetscErrorCode MatCreateDense(MPI_Comm, PetscInt, PetscInt, PetscInt, PetscInt, PetscScalar[], Mat *); PETSC_ERR_SUP on
+   more than one rank */
+PERMON_EXTERN PetscErrorCode MatCreateDense(MPI_Comm comm, PetscInt m, PetscInt n, PetscInt M, PetscInt N, PetscScalar data[], Mat *A);
+/* petscmat.h: PetscErrorCode MatDenseSetLDA(Mat, PetscInt) / MatDenseGetLDA(Mat, PetscInt *): the caller's leading dimension */
+PERMON_EXTERN PetscErrorCode MatDenseSetLDA(Mat A, PetscInt lda);
+PERMON_EXTERN PetscErrorCode MatDenseGetLDA(Mat A, PetscInt *lda);
+/* device form of a dense matrix: leading dimension of the array the kernels read, whether that is the caller's device array, rows per
+   CTA, and the column chunk of the split-column variant (0: one thread per row) */
+PERMON_EXTERN PetscErrorCode MatB200GetDenseInfo(Mat A, int64_t *lda, PetscBool *adopted, PetscInt *rows_per_block, PetscInt *split_columns);
 /* include/permonmat.h:36, src/mat/impls/onerow/onerow.c:97: the 1 x n matrix a^T */
 PERMON_EXTERN PetscErrorCode MatCreateOneRow(Vec a, Mat *A_new);
 /* include/permonmat.h:28, src/mat/impls/composite/matprod.c:42: implicit product mats[nmat-1]*...*mats[0] (nmat <= 2) */
@@ -212,7 +230,7 @@ PERMON_EXTERN PetscErrorCode MatB200GetHostSplit(Mat A, const PetscInt **dia, co
                                                  const PetscInt **oia, const PetscInt **oja, const PetscScalar **oa, const PetscInt **orow);
 /* device storage introspection: kind 0/1/2 = CSR (tile-streamed / vector / TMA-staged), 3 = packed dictionary-coded tiles;
    stream_bytes = bytes one SpMV reads for the matrix itself (diagonal + off-diagonal block); coded_tiles / tiles of the packed form.
-   Uploads a row-partitioned matrix if it is not on the device yet. */
+   Uploads a row-partitioned matrix if it is not on the device yet.  Dense matrices: kind 6, stream_bytes = 8 m n, tiles = row blocks. */
 PERMON_EXTERN PetscErrorCode MatB200GetStorageInfo(Mat A, PetscInt *kind, PetscReal *stream_bytes, PetscInt *coded_tiles, PetscInt *tiles);
 /* like MatCreateMPIAIJWithArrays, but di / dj / da are CUDA device pointers (int32 row pointer, GLOBAL column ids, fp64 values) of the
    device the library runs on.  The arrays must be complete when the call is made (device-synchronised, or written on the stream of

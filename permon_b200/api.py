@@ -373,6 +373,73 @@ def MatCreateAIJFromDeviceTensors(ia, ja, a, ncols_local=None, comm=None):
     return A
 
 
+def _colmajor_lda(shape, strides):
+    """leading dimension (in elements) when a 2-D array with these element strides is column-major with lda >= m, else None"""
+    m, n = shape
+    if m > 1 and strides[0] != 1:
+        return None
+    lda = strides[1] if n > 1 else max(m, 1)
+    return lda if lda >= max(m, 1) else None
+
+
+def MatCreateDense(arr, comm=None):
+    """MatCreateSeqDense (MatCreateDense on one rank): a 2-D float64 NumPy array in any order.  A column-major array (or a column-major view
+    with a leading dimension, e.g. big[:m, :] of a Fortran-ordered big) is handed over as it is, anything else is copied column-major first.
+    The library uploads it at the first use; the array is kept alive with the matrix."""
+    arr = np.asarray(arr, dtype=np.float64)
+    if arr.ndim != 2:
+        raise ValueError(f"a 2-D array is required (got shape {arr.shape})")
+    lda = _colmajor_lda(arr.shape, tuple(s // 8 for s in arr.strides)) if all(s % 8 == 0 and s >= 0 for s in arr.strides) else None
+    if lda is None:
+        arr = np.asfortranarray(arr)
+        lda = max(arr.shape[0], 1)
+    m, n = arr.shape
+    A = C.c_void_p()
+    call("MatCreateDense", comm or world(), C.c_int(m), C.c_int(n), C.c_int(DECIDE), C.c_int(DECIDE), C.c_void_p(arr.ctypes.data), C.byref(A))
+    _keep(A, arr)
+    if lda != max(m, 1):
+        call("MatDenseSetLDA", A, C.c_int(lda))
+    return A
+
+
+def MatCreateDenseFromTensor(t, comm=None):
+    """MatCreateSeqDenseCUDA from a 2-D torch CUDA float64 tensor on the library's device.  A column-major tensor (stride(0) == 1, stride(1)
+    = lda >= m) is adopted without a copy when its base is 16-byte aligned and lda is even: every product reads the tensor, so in-place
+    changes show in the next MatMult.  Otherwise one column-major device copy is made here and handed over instead.  A symmetric Hessian
+    in row-major order is already its own column-major form: pass H.T (a view) to have it adopted.  The tensor is kept alive with the
+    matrix."""
+    import torch
+    if not isinstance(t, torch.Tensor) or t.device.type != "cuda" or t.dtype != torch.float64 or t.dim() != 2:
+        raise TypeError("a 2-D torch CUDA float64 tensor is required")
+    lda = _colmajor_lda(tuple(t.shape), t.stride())
+    if lda is None:
+        t = t.t().contiguous().t()
+        lda = max(t.shape[0], 1)
+    m, n = t.shape
+    # the tensor was written on torch's current stream: the library reads it on its own stream
+    torch.cuda.current_stream(t.device).synchronize()
+    A = C.c_void_p()
+    call("MatCreateSeqDenseCUDA", comm or world(), C.c_int(m), C.c_int(n), C.c_void_p(t.data_ptr()), C.byref(A))
+    _keep(A, t)
+    if lda != max(m, 1):
+        call("MatDenseSetLDA", A, C.c_int(lda))
+    return A
+
+
+def MatDenseGetLDA(A) -> int:
+    lda = C.c_int()
+    call("MatDenseGetLDA", A, C.byref(lda))
+    return lda.value
+
+
+def MatDenseGetInfo(A):
+    """MatB200GetDenseInfo: leading dimension the kernels read with, whether the caller's device array is read in place, rows per CTA,
+    column chunk of the split-column variant (0: one thread per row)"""
+    lda, adopted, rpb, split = C.c_int64(), C.c_int(), C.c_int(), C.c_int()
+    call("MatB200GetDenseInfo", A, C.byref(lda), C.byref(adopted), C.byref(rpb), C.byref(split))
+    return dict(lda=lda.value, adopted=bool(adopted.value), rows_per_block=rpb.value, split_columns=split.value)
+
+
 FORM_PARTS = {"scalars": 0, "st_masks": 1, "st_pid": 2, "st_pats": 3, "pk_blob": 4, "pk_off": 5, "csr_ia": 6, "csr_ja": 7, "csr_a": 8,
               "ell_val": 9, "ell_col": 10, "ell_len": 11, "ell_lt": 12, "ell_off": 13, "rows": 14}
 FORM_OFFDIAG = 16
@@ -448,7 +515,8 @@ def MatGetHostSplit(A, m):
 
 
 def MatStorageInfo(A):
-    """Device storage of an AIJ matrix: kind (3 = packed dictionary-coded tiles), matrix bytes streamed per SpMV, coded / all tiles."""
+    """Device storage of an AIJ or dense matrix: kind (3 = packed dictionary-coded tiles, 6 = dense), matrix bytes streamed per SpMV, coded / all
+    tiles (dense: row blocks)."""
     kind, coded, tiles = C.c_int(), C.c_int(), C.c_int()
     nbytes = C.c_double()
     call("MatB200GetStorageInfo", A, C.byref(kind), C.byref(nbytes), C.byref(coded), C.byref(tiles))
@@ -740,12 +808,13 @@ class Solved:
     pass
 
 
-def solve_problem(pr, qps_type=None, options: str = "", monitor=None, keep=False, device_arrays=None, device_input=None):
+def solve_problem(pr, qps_type=None, options: str = "", monitor=None, keep=False, device_arrays=None, device_input=None, dense=False):
     """Build QP + QPS for a permon_b200.problems.QPProblem through the C ABI, solve, return a result object.
 
     `options` is a PETSc-style option string ("-qps_rtol 1e-8 -qps_mpgp_expansion_type gf ...").
     `device_input`: "keep" builds the AIJ matrices from torch CUDA tensors (MatCreateAIJFromDeviceTensors), "zero" does the same and
-    zeroes the tensors right after each constructor returns."""
+    zeroes the tensors right after each constructor returns.
+    `dense`: the Hessian (both factors of a product Hessian) is built as a dense matrix from the problem's CSR (MatCreateDense)."""
     if device_input:
         import torch
 
@@ -759,6 +828,12 @@ def solve_problem(pr, qps_type=None, options: str = "", monitor=None, keep=False
             return M
     else:
         MatCreateAIJ = globals()["MatCreateAIJ"]
+    MatCreateH = MatCreateAIJ
+    if dense:
+        import scipy.sparse as sp
+
+        def MatCreateH(ia, ja, a, ncols_local=None):
+            return MatCreateDense(sp.csr_matrix((a, ja, ia), shape=(len(ia) - 1, ncols_local)).toarray(order="F"))
     options_clear()
     if options:
         call("PetscOptionsInsertString", None, options.encode())
@@ -766,11 +841,11 @@ def solve_problem(pr, qps_type=None, options: str = "", monitor=None, keep=False
     x_host = np.ascontiguousarray(pr.x0, dtype=np.float64).copy()
     b_host = np.ascontiguousarray(pr.b, dtype=np.float64)
     ncols = pr.n
-    A1 = MatCreateAIJ(pr.ia, pr.ja, pr.a, ncols_local=(pr.meta.get("d") if pr.second is not None else ncols))
+    A1 = MatCreateH(pr.ia, pr.ja, pr.a, ncols_local=(pr.meta.get("d") if pr.second is not None else ncols))
     mats = [A1]
     A = A1
     if pr.second is not None:
-        A2 = MatCreateAIJ(pr.second[0], pr.second[1], pr.second[2], ncols_local=pr.n)
+        A2 = MatCreateH(pr.second[0], pr.second[1], pr.second[2], ncols_local=pr.n)
         A = MatCreateProd([A2, A1])   # product = mats[1]*mats[0] = A1 * A2
         mats += [A2, A]
     b = VecFromArray(b_host)

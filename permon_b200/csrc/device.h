@@ -164,7 +164,8 @@ struct CsrDev {
   int64_t       nnz_alloc = 0;     // elements of ja / a that may be read (allocation incl. padding)
   int           ia_alloc = 0;      // entries of ia that may be read
   int           stages = 2;        // shared-memory stages of the TMA kernel
-  int           kind   = 0;        // 0: tile-streamed plain loads, 1: vector (W lanes per row), 2: TMA-staged CSR tiles, 3: TMA-staged packed tiles, 4: stencil windows
+  int           kind   = 0;        // 0: tile-streamed plain loads, 1: vector (W lanes per row), 2: TMA-staged CSR tiles, 3: TMA-staged packed tiles, 4: stencil windows,
+                                   // 5: tile-ELL, 6: dense column-major
   // packed tiles (kind 3): blob + tile directory (offsets in 16-byte units); the raw CSR arrays are then absent
   const unsigned char *pk     = nullptr;
   const unsigned      *pk_off = nullptr;
@@ -185,6 +186,14 @@ struct CsrDev {
   const int    *ell_lt  = nullptr;     // [ntiles] longest row of each tile
   const int64_t *ell_off = nullptr;    // [ntiles] first element of each tile in ell_val / ell_col
   int64_t       ell_elems = 0;         // elements stored (padding included)
+  // dense matrices (kind 6): column-major, entry (i, j) at dn_a[i + j * dn_lda]; dn_a is 16-byte aligned and dn_lda even, so every
+  // column segment can be staged with bulk copies.  dn_rpb rows per CTA (one consumer thread per row); dn_split > 0: split-column
+  // variant with column chunks of dn_split columns, partial sums in dn_part [nchunks][n]
+  const double *dn_a     = nullptr;
+  int64_t       dn_lda   = 0;
+  int           dn_rpb   = 0;
+  int           dn_split = 0;
+  double       *dn_part  = nullptr;
   int           W      = 32;
   int           tile_cap = 0;      // max nnz of a 256-row tile (stream kind)
   int           grid   = 0;        // persistent grid size (fixed => reproducible reductions)
@@ -360,6 +369,8 @@ int  recode_stencil_window_dev(CsrDev &A, int m, const int *d_ia, const int *d_j
 // want_diag, the diagonal block [c0, c0 + ncols) as a padded device CSR with local columns (library-owned, released with dfree)
 int  split_rows_dev(int m, const int *d_ia, const int *d_ja, const double *d_a, int c0, int ncols, bool want_diag, int **dia, int **dja, double **da,
                     OffDiagEntries &off);
+// dense form (kind 6): rows per CTA and split-column chunk from (m, n, SM count) only, so that grids and reductions are reproducible
+void dense_config(CsrDev &A);
 int  elementwise_grid();
 int  fused_C_grid(int n);   // CTAs of K_C for n local rows (K_A adds that many partial sums of g.p)
 int  max_red_blocks();

@@ -1698,6 +1698,210 @@ int csr_to_tile_ell_widths(CsrDev &A, const std::vector<int> &tile_maxrow)
   return 0;
 }
 
+// ---- dense column-major matrices (kind 6) ----------------------------------------------------------------------------------------
+// One CTA owns a block of R = A.dn_rpb consecutive rows, one consumer thread per row.  A producer warp streams the block's column
+// segments (R * 8 contiguous bytes each, stride lda) with bulk copies into a ring of shared-memory stages of kc columns (plus the kc
+// entries of x), guarded by mbarriers; consumers read smem[j][t] (conflict-free) and x[j] as a broadcast.  Each row's products are
+// added in ascending column order with fma, starting from 0 -- the order of the storage-order CSR kernels (k_spmv_ell, k_spmv_tma), so
+// a dense MatMult is bit-identical to the AIJ matrix that stores every entry.  Row blocks are walked by a grid of min(blocks,
+// max_red_blocks()) CTAs, a function of (m, n, SM count) only, so reductions of the epilogue are reproducible.  Epi::reverse()
+// (serpentine sweeps) is ignored: the order of the row blocks changes nothing in a row's sum.
+static constexpr int DN_MAX_R = 512;
+static constexpr int DN_MAX_STAGES = 8;
+struct DnLayout {
+  int kc, stage_bytes, nstages;
+};
+static DnLayout dense_layout(int R)
+{
+  DnLayout L;
+  L.kc = (32768 / (R * 8)) & ~1;   // ~32 KB of matrix per stage
+  if (L.kc > 32) L.kc = 32;
+  if (L.kc < 2) L.kc = 2;
+  L.stage_bytes = (L.kc * R * 8 + L.kc * 8 + 127) & ~127;
+  L.nstages     = (200 * 1024) / L.stage_bytes;   // tens of KB in flight per SM even when R is small
+  if (L.nstages > DN_MAX_STAGES) L.nstages = DN_MAX_STAGES;
+  if (L.nstages < 2) L.nstages = 2;
+  return L;
+}
+
+template <class Epi>
+__global__ void __launch_bounds__(DN_MAX_R + 32) k_dense(CsrDev A, const double *__restrict__ x, Epi epi, int kc, int stage_bytes, int nstages)
+{
+  pdl_enter();
+  if (!epi.active()) return;
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  __shared__ uint64_t full_bar[DN_MAX_STAGES], empty_bar[DN_MAX_STAGES];
+  const int R = A.dn_rpb, ncw = R / 32;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int nblk = (A.n + R - 1) / R, nchunk = (A.ncols + kc - 1) / kc;
+  typename Epi::Acc acc;
+  epi.init(acc);
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < nstages; s++) {
+      mbar_init(&full_bar[s], 1);
+      mbar_init(&empty_bar[s], ncw);
+    }
+    mbar_fence_init();
+  }
+  __syncthreads();
+
+  if (warp == ncw) {
+    // ------------------------------ producer warp ------------------------------
+    const typename Epi::Gather g = epi.gather(x);
+    int      s = 0, filled = 0;
+    uint32_t ph = 0;
+    for (int blk = blockIdx.x; blk < nblk; blk += gridDim.x) {
+      const int      r0 = blk * R, nrow = min(R, A.n - r0);
+      const uint32_t seg = (uint32_t)(nrow & ~1) * 8u;   // bulk copies move 16-byte granules: an odd last row is stored by the warp
+      for (int c = 0; c < nchunk; c++) {
+        if (filled >= nstages) mbar_wait(&empty_bar[s], ph ^ 1u);
+        else filled++;
+        double   *ms = (double *)(smem_raw + (size_t)s * stage_bytes);
+        double   *xs = ms + (size_t)kc * R;
+        const int j0 = c * kc, nc = min(kc, A.ncols - j0);
+        for (int jj = lane; jj < nc; jj += 32) {
+          xs[jj] = g.ld(x + j0 + jj);
+          if (nrow & 1) ms[(size_t)jj * R + nrow - 1] = __ldg(A.dn_a + (size_t)r0 + (size_t)(j0 + jj) * A.dn_lda + nrow - 1);
+        }
+        fence_proxy_async_smem();
+        __syncwarp();
+        if (lane == 0) mbar_arrive_expect_tx(&full_bar[s], seg * (uint32_t)nc);
+        __syncwarp();
+        if (seg)
+          for (int jj = lane; jj < nc; jj += 32) bulk_g2s(ms + (size_t)jj * R, A.dn_a + (size_t)r0 + (size_t)(j0 + jj) * A.dn_lda, seg, &full_bar[s]);
+        if (++s == nstages) {
+          s  = 0;
+          ph ^= 1u;
+        }
+      }
+    }
+  } else {
+    // ------------------------------ consumer warps: one thread per row ------------------------------
+    const int t = threadIdx.x;
+    int       s = 0;
+    uint32_t  ph = 0;
+    for (int blk = blockIdx.x; blk < nblk; blk += gridDim.x) {
+      const int r0 = blk * R, nrow = min(R, A.n - r0);
+      double    sum = 0.0;
+      for (int c = 0; c < nchunk; c++) {
+        mbar_wait(&full_bar[s], ph);
+        const double *ms = (const double *)(smem_raw + (size_t)s * stage_bytes);
+        const double *xs = ms + (size_t)kc * R;
+        const int     nc = min(kc, A.ncols - c * kc);
+        if (t < nrow) {
+          const double *mt = ms + t;
+          int           jj = 0;
+          for (; jj + 2 <= nc; jj += 2) {
+            const double2 xv = *reinterpret_cast<const double2 *>(xs + jj);
+            sum = fma(mt[(size_t)jj * R], xv.x, sum);
+            sum = fma(mt[(size_t)(jj + 1) * R], xv.y, sum);
+          }
+          if (jj < nc) sum = fma(mt[(size_t)jj * R], xs[jj], sum);
+        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&empty_bar[s]);
+        if (++s == nstages) {
+          s  = 0;
+          ph ^= 1u;
+        }
+      }
+      if (t < nrow) epi.row(r0 + t, sum, acc);
+    }
+  }
+  epi.finalize(acc);
+}
+
+// Split-column variant for wide matrices (n > 64 m: too few rows to fill the GPU with one thread per row).  Pass 1: CTA (row block,
+// chunk) sums the products of columns [c * S, (c + 1) * S) of each of its rows in ascending column order with fma from 0 into
+// dn_part[c][r].  Pass 2: row r adds its chunk sums in chunk order, s = ((p_0 + p_1) + p_2) + ..., starting from 0.0, and runs the
+// epilogue.  The chunk width S depends on (m, n, SM count) only: deterministic, but not the order of a CSR row sum.
+template <class Epi>
+__global__ void __launch_bounds__(NT) k_dense_part(CsrDev A, const double *__restrict__ x, Epi epi)
+{
+  pdl_enter();
+  if (!epi.active()) return;
+  const typename Epi::Gather g = epi.gather(x);
+  const int nrb = (A.n + (int)blockDim.x - 1) / (int)blockDim.x;
+  const int rb = blockIdx.x % nrb, c = blockIdx.x / nrb;
+  const int r = rb * blockDim.x + threadIdx.x;
+  if (r >= A.n) return;
+  const int     j0 = c * A.dn_split, j1 = min(A.ncols, j0 + A.dn_split);
+  const double *col = A.dn_a + r;
+  double        s = 0.0;
+  int           j = j0;
+  for (; j + 8 <= j1; j += 8) {
+    double v[8], xv[8];
+#pragma unroll
+    for (int u = 0; u < 8; u++) {
+      v[u]  = __ldcs(col + (size_t)(j + u) * A.dn_lda);
+      xv[u] = g.ld(x + j + u);
+    }
+#pragma unroll
+    for (int u = 0; u < 8; u++) s = fma(v[u], xv[u], s);
+  }
+  for (; j < j1; j++) s = fma(__ldcs(col + (size_t)j * A.dn_lda), g.ld(x + j), s);
+  A.dn_part[(size_t)c * A.n + r] = s;
+}
+template <class Epi>
+__global__ void __launch_bounds__(NT) k_dense_combine(CsrDev A, Epi epi)
+{
+  pdl_enter();
+  if (!epi.active()) return;
+  typename Epi::Acc acc;
+  epi.init(acc);
+  const int nch = (A.ncols + A.dn_split - 1) / A.dn_split;
+  for (int r = blockIdx.x * NT + threadIdx.x; r < A.n; r += gridDim.x * NT) {
+    double s = 0.0;
+    for (int c = 0; c < nch; c++) s += __ldcg(A.dn_part + (size_t)c * A.n + r);
+    epi.row(r, s, acc);
+  }
+  epi.finalize(acc);
+}
+
+void dense_config(CsrDev &A)
+{
+  const int64_t m = A.n, n = A.ncols, sm = g_ctx.sm_count > 0 ? g_ctx.sm_count : 148;
+  A.kind     = 6;
+  A.dn_split = 0;
+  if (n > 64 * m && m > 0) {
+    // wide: R = the rows rounded up to a warp (at most NT), ~4 CTAs per SM over the column chunks, chunks a multiple of 64 columns
+    const int64_t R = std::min<int64_t>(NT, (m + 31) / 32 * 32), nrb = (m + R - 1) / R;
+    int64_t       nch = std::max<int64_t>(1, (4 * sm + nrb - 1) / nrb);
+    int64_t       S = (n + nch - 1) / nch;
+    S = std::max<int64_t>(64, (S + 63) / 64 * 64);
+    A.dn_rpb   = (int)R;
+    A.dn_split = (int)S;
+    return;
+  }
+  // one thread per row: the smallest R (a multiple of 32, at most DN_MAX_R) that covers the rows in the fewest waves of one CTA per SM
+  const int64_t waves = std::max<int64_t>(1, (m + DN_MAX_R * sm - 1) / (DN_MAX_R * sm));
+  int64_t       R = (m + 32 * sm * waves - 1) / (32 * sm * waves) * 32;
+  A.dn_rpb = (int)std::min<int64_t>(DN_MAX_R, std::max<int64_t>(32, R));
+}
+
+template <class Epi>
+static void launch_dense(const CsrDev &A, const double *x, const Epi &epi)
+{
+  if (A.dn_split > 0) {
+    const int nrb = (A.n + A.dn_rpb - 1) / A.dn_rpb, nch = (A.ncols + A.dn_split - 1) / A.dn_split;
+    launch_k(k_dense_part<Epi>, nrb * nch, A.dn_rpb, 0, A, x, epi);
+    int grid = (A.n + NT - 1) / NT;
+    if (grid > max_red_blocks()) grid = max_red_blocks();
+    launch_k(k_dense_combine<Epi>, grid, NT, 0, A, epi);
+    return;
+  }
+  const DnLayout L = dense_layout(A.dn_rpb);
+  const size_t   smem = (size_t)L.stage_bytes * L.nstages;
+  static size_t  attr_smem = 0;
+  if (smem > attr_smem) {
+    cudaFuncSetAttribute(k_dense<Epi>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    attr_smem = smem;
+  }
+  int grid = (A.n + A.dn_rpb - 1) / A.dn_rpb;
+  if (grid > max_red_blocks()) grid = max_red_blocks();
+  launch_k(k_dense<Epi>, grid, A.dn_rpb + 32, smem, A, x, epi, L.kc, L.stage_bytes, L.nstages);
+}
+
 template <class Epi, class = void>
 struct EpiHasStaged : std::false_type {};
 template <class Epi>
@@ -1928,6 +2132,18 @@ static int launch_sd(const CsrDev &A, const double *x, const Epi &epi, TileOrder
   }
 }
 
+// epilogues that merge ghost columns (multi-GPU instantiations): never paired with a dense matrix, which lives on one rank
+template <int MODE, bool GHOST>
+struct EpiAT;
+template <int MODE, bool GHOST>
+struct EpiA2T;
+template <class Epi>
+struct EpiGhostMerge : std::false_type {};
+template <int MODE>
+struct EpiGhostMerge<EpiAT<MODE, true>> : std::true_type {};
+template <int MODE>
+struct EpiGhostMerge<EpiA2T<MODE, true>> : std::true_type {};
+
 template <class Epi>
 static int launch_spmv(const CsrDev &A, const double *x, const Epi &epi, int family, double bytes, TileOrder ord = TileOrder())
 {
@@ -1935,6 +2151,13 @@ static int launch_spmv(const CsrDev &A, const double *x, const Epi &epi, int fam
   if (A.n == 0) {
     // still run one CTA so that reductions publish their (identity) record
     k_spmv_vector<Epi, 32><<<1, NT, 0, g_ctx.stream>>>(A, x, epi);
+  } else if (A.kind == 6) {
+    if constexpr (EpiGhostMerge<Epi>::value) {
+      set_error("internal: a dense matrix with ghost columns");
+      return 76;
+    } else {
+      launch_dense(A, x, epi);
+    }
   } else if (A.kind == 5) {
     launch_ell(A, x, epi);
   } else if (A.kind == 4) {
@@ -1980,6 +2203,7 @@ double csr_stream_bytes(const CsrDev &A)
 {
   if (A.kind == 3 || A.kind == 4) return (double)A.pk_bytes;
   if (A.kind == 5) return 12.0 * (double)A.ell_elems + 4.0 * A.n;
+  if (A.kind == 6) return 8.0 * (double)A.n * (double)A.ncols;
   return 12.0 * (double)A.nnz + 4.0 * (A.n + 1);
 }
 
@@ -2552,8 +2776,8 @@ struct EpiPower {
 };
 int k_power_step(const CsrDev &A, const double *w, double s, double *y, RedBuf rb)
 {
-  if (A.kind != 3 && A.kind != 4) {
-    set_error("internal: fused power step needs a packed matrix");
+  if (A.kind != 3 && A.kind != 4 && A.kind != 6) {
+    set_error("internal: fused power step needs a packed or dense matrix");
     return 76;
   }
   EpiPower e{w, s, y, rb};

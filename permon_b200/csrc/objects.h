@@ -126,7 +126,8 @@ struct HaloPlan {
 };
 
 enum MatKind { MK_AIJ = 0, MK_ONEROW, MK_PROD, MK_PENALIZED, MK_PROJ /* P = I - G'(GG')^-1 G of a QPPF */, MK_DENSEROWS /* m x n dense rows on the device */,
-               MK_DUMMY /* MatCreateDummy of the implicit orthonormalisation (permonmatorth.c:176-192): no MatMult; `A` = the matrix it stands for */ };
+               MK_DUMMY /* MatCreateDummy of the implicit orthonormalisation (permonmatorth.c:176-192): no MatMult; `A` = the matrix it stands for */,
+               MK_DENSE /* column-major m x n (MATSEQDENSE / MATSEQDENSECUDA), device form in Ad (kind 6) */ };
 
 struct _p_Mat : PObj {
   MatKind  kind = MK_AIJ;
@@ -155,6 +156,12 @@ struct _p_Mat : PObj {
   QPPF   pf = nullptr;
   double rho = 0.0;
   int    proj_mode = 0;   // PROJ: 0 P = I - Q (QPPFCreateP), 1 Q (QPPFCreateQ), 2 G^T G (QPPFCreateGtG)
+  // DENSE: the caller's array (host, or device when dn_src_dev) and its leading dimension until the first use (mat_ensure_device), which
+  // adopts a suitably aligned device array or makes the library's padded device copy (dn_own)
+  const double *dn_src = nullptr;
+  int64_t       dn_src_lda = 0;
+  bool          dn_src_dev = false, dn_ready = false, dn_adopted = false;
+  double       *dn_own = nullptr;
   // cached extreme eigenvalue (PetscObjectComposedData in the reference)
   ~_p_Mat() override;
 };

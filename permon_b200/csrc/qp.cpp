@@ -425,6 +425,17 @@ PetscErrorCode QPPFSetUp(QPPF cp)
     // row-partitioned AIJ equality matrix (several GPUs): re-distributed by columns into dense rows (shim.cpp: mat_eqrows_dense)
     PB_CHK(mat_eqrows_dense(G, &cp->Bd));
     cp->Bd_owned = false;
+  } else if (G->kind == MK_DENSE) {
+    // column-major m x n (m <= PB_MAXEQ_ALL, checked above) -> the row-major [m][n] rows: one strided device-to-device copy per row
+    PB_CHK(mat_ensure_device(G));
+    const int     m = G->m, n = G->n;
+    const int64_t lda = G->Ad.dn_lda;
+    PB_CUDA(cudaMalloc(&cp->Bd, sizeof(double) * std::max<size_t>((size_t)m * n, 1)));
+    for (int r = 0; r < m && n > 0; r++)
+      PB_CUDA(cudaMemcpy2DAsync(cp->Bd + (size_t)r * n, sizeof(double), G->Ad.dn_a + r, sizeof(double) * (size_t)lda, sizeof(double), (size_t)n,
+                                cudaMemcpyDeviceToDevice, ctx().stream));
+    PB_CUDA(cudaStreamSynchronize(ctx().stream));
+    cp->Bd_owned = true;
   } else if (G->kind == MK_AIJ) {
     if (G->comm->size > 1) return err(PETSC_ERR_SUP, "a row-partitioned AIJ equality matrix may have at most %d rows", PB_MAXEQ_ALL);
     const int        m = G->m, n = G->n;

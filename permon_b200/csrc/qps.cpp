@@ -550,8 +550,9 @@ struct MpgpImpl : QPSImpl {   // QPS_MPGP mpgpimpl.h:5-38
       if (A->pf && A->pf->implicit_orth) return false;                 // penalised term Q = B'(BB')^-1 B: the coarse solve sits between the two rank-m halves
       A = A->A;
     }
-    if (A->kind == MK_PROD) return A->M1->kind == MK_AIJ && A->M2->kind == MK_AIJ && A->comm->size == 1;
-    return A->kind == MK_AIJ;
+    auto one_gpu = [](Mat F) { return F->kind == MK_AIJ || F->kind == MK_DENSE; };   // dense matrices live on one rank only
+    if (A->kind == MK_PROD) return one_gpu(A->M1) && one_gpu(A->M2) && A->comm->size == 1;
+    return A->kind == MK_AIJ || A->kind == MK_DENSE;
   }
   int engine_init(QPS qps);
   int solve_fused(QPS qps);
@@ -610,7 +611,7 @@ PetscErrorCode MpgpImpl::setup(QPS qps)
   if (fallback || fallback2) nw = (explengthtype != QPS_MPGP_EXPANSION_LENGTH_BB) ? 9 : 10;
   else if (explengthtype == QPS_MPGP_EXPANSION_LENGTH_BB) nw = 9;
   const bool fused = fused_eligible(qps);
-  if (driver == "fused" && !fused) return err(PETSC_ERR_SUP, "-qps_mpgp_b200_driver fused needs expansion std/fixed, no fallback and an AIJ (or product-of-AIJ) Hessian");
+  if (driver == "fused" && !fused) return err(PETSC_ERR_SUP, "-qps_mpgp_b200_driver fused needs expansion std/fixed, no fallback and an AIJ or dense Hessian (or a product of such)");
   {
     PhaseTimer pt("MPGP set-up: work vectors");
     PB_CHK(set_work(qps, nw));

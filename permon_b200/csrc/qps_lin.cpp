@@ -52,7 +52,7 @@ struct KspImpl : QPSImpl {
   }
   // QPSSolve_KSP (qpsksp.c:137-153) -> KSPSolve on KSPCG / PCNONE / KSP_NORM_UNPRECONDITIONED / non-zero initial guess
   // (QPSCreate_KSP qpsksp.c:232-253); the stopping test is the QPS one (QPSKSPConverged_KSP qpsksp.c:5-14).
-  // Fused form for a packed AIJ Hessian on one GPU (-qps_ksp_b200_driver generic switches it off): per iteration ONE SpMV kernel that
+  // Fused form for a packed AIJ or a dense Hessian on one GPU (-qps_ksp_b200_driver generic switches it off): per iteration ONE SpMV kernel that
   // also reduces p.Ap (the power-method skeleton, kernels.cu: EpiPower with s = 1), ONE update kernel (x += a p, r -= a w, r.r) and the
   // direction update -- 3 kernels and 2 host round trips instead of 7 and 4, 11 vector passes instead of 15.  Same recurrence, same
   // stopping test; the products p.w and r.r are summed by other kernels than in the un-fused form (deterministic, different order).
@@ -62,9 +62,9 @@ struct KspImpl : QPSImpl {
     std::string d = "auto";
     options_string(qps->prefix, "-qps_ksp_b200_driver", &d);
     if (d == "generic") return false;
-    if (A->kind != MK_AIJ || A->comm->size != 1 || A->m != A->n || A->eq_host) return false;
+    if ((A->kind != MK_AIJ && A->kind != MK_DENSE) || A->comm->size != 1 || A->m != A->n || A->eq_host) return false;
     if (mat_ensure_device(A)) return false;
-    return A->Ad.kind == 3 || A->Ad.kind == 4;
+    return A->Ad.kind == 3 || A->Ad.kind == 4 || A->Ad.kind == 6;
   }
   PetscErrorCode solve_fused(QPS qps)
   {

@@ -979,6 +979,10 @@ _p_Mat::~_p_Mat()
     pb::dfree(Ad.ell_off);
   }
   if (kind == MK_DENSEROWS || eq_host) pb::dfree(rows_d);
+  if (kind == MK_DENSE) {
+    pb::dfree(dn_own);
+    pb::dfree(Ad.dn_part);
+  }
   delete eq_host;
   if (kind == MK_AIJ) {
     pb::dfree(Ao.ia);
@@ -1597,6 +1601,41 @@ static int halo_device_setup(Mat A, const std::vector<int> &orow)
   return 0;
 }
 
+// First use of a dense matrix: a device array whose base is 16-byte aligned and whose lda is even (every column start 16-byte aligned,
+// what the bulk copies of k_dense need) is adopted as it is; anything else -- host arrays, odd lda, offset device pointers -- goes into
+// one library-owned device copy with an even lda.
+static int dense_ensure_device(Mat A)
+{
+  if (A->dn_ready) return 0;
+  PB_CHK(dev_init());
+  PhaseTimer     pt("dense matrix: adopt / upload");
+  cudaStream_t   s = ctx().stream;
+  const int64_t  m = A->m, n = A->n, lda = A->dn_src_lda;
+  pb::CsrDev    &C = A->Ad;
+  C.n     = (int)m;
+  C.ncols = (int)n;
+  C.nnz   = m * n;
+  if (A->dn_src_dev && (((uintptr_t)A->dn_src) & 15) == 0 && lda % 2 == 0) {
+    C.dn_a        = A->dn_src;
+    C.dn_lda      = lda;
+    A->dn_adopted = true;
+  } else {
+    const int64_t ldp = (m + 1) / 2 * 2;
+    PB_CHK(dmalloc(&A->dn_own, (size_t)std::max<int64_t>(ldp * n, 1)));
+    if (m > 0 && n > 0)
+      PB_CUDA(cudaMemcpy2DAsync(A->dn_own, (size_t)ldp * 8, A->dn_src, (size_t)lda * 8, (size_t)m * 8, (size_t)n,
+                                A->dn_src_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s));
+    if (ldp > m && n > 0) PB_CUDA(cudaMemset2DAsync(A->dn_own + m, (size_t)ldp * 8, 0, 8, (size_t)n, s));   // the pad row is never summed
+    PB_CUDA(cudaStreamSynchronize(s));   // the host array may be pageable and may change after this call
+    C.dn_a   = A->dn_own;
+    C.dn_lda = ldp;
+  }
+  pb::dense_config(C);
+  if (C.dn_split > 0) PB_CHK(dmalloc(&C.dn_part, (size_t)std::max<int64_t>(m * ((n + C.dn_split - 1) / C.dn_split), 1)));
+  A->dn_ready = true;
+  return 0;
+}
+
 namespace pb {
 int mat_ensure_device(Mat A)
 {
@@ -1605,6 +1644,7 @@ int mat_ensure_device(Mat A)
     return mat_ensure_device(A->M2);
   }
   if (A->kind == MK_PENALIZED) return mat_ensure_device(A->A);
+  if (A->kind == MK_DENSE) return dense_ensure_device(A);
   if (A->kind != MK_AIJ || !A->halo || !A->halo->host) return 0;
   HaloPlan            *H = A->halo;
   HaloPlan::HostSplit *S = H->host;
@@ -1681,8 +1721,15 @@ PetscErrorCode MatB200GetHostSplit(Mat A, const PetscInt **dia, const PetscInt *
 
 PetscErrorCode MatB200GetStorageInfo(Mat A, PetscInt *kind, PetscReal *stream_bytes, PetscInt *coded_tiles, PetscInt *tiles)
 {
-  if (!A || A->kind != MK_AIJ) return err(PETSC_ERR_ARG_WRONG, "MatB200GetStorageInfo: AIJ matrix expected");
+  if (!A || (A->kind != MK_AIJ && A->kind != MK_DENSE)) return err(PETSC_ERR_ARG_WRONG, "MatB200GetStorageInfo: AIJ or dense matrix expected");
   PB_CHK(pb::mat_ensure_device(A));
+  if (A->kind == MK_DENSE) {
+    if (kind) *kind = A->Ad.kind;
+    if (stream_bytes) *stream_bytes = pb::csr_stream_bytes(A->Ad);
+    if (coded_tiles) *coded_tiles = 0;
+    if (tiles) *tiles = A->Ad.dn_rpb ? (A->Ad.n + A->Ad.dn_rpb - 1) / A->Ad.dn_rpb : 0;   // row blocks
+    return 0;
+  }
   if (kind) *kind = A->Ad.kind;
   if (stream_bytes) *stream_bytes = pb::csr_stream_bytes(A->Ad) + (A->halo ? pb::csr_stream_bytes(A->Ao) : 0.0);
   if (coded_tiles) *coded_tiles = (PetscInt)A->Ad.pk_coded;
@@ -1808,6 +1855,65 @@ PetscErrorCode MatB200CreateAIJWithDeviceArrays(MPI_Comm comm, PetscInt m, Petsc
   if (!ierr && cudaStreamSynchronize(s) != cudaSuccess) ierr = err(PETSC_ERR_GPU, "%s", cudaGetErrorString(cudaGetLastError()));
   if (ierr) return fail(ierr);
   *mat = A;
+  return 0;
+}
+
+// ---- dense matrices (MATSEQDENSE / MATSEQDENSECUDA): column-major, entry (i, j) at data[i + j * lda], lda = m until MatDenseSetLDA --------
+static int dense_create(MPI_Comm comm, PetscInt m, PetscInt n, const PetscScalar *data, bool dev, Mat *mat)
+{
+  if (!mat) return err(PETSC_ERR_ARG_NULL, "null Mat pointer");
+  if (m < 0 || n < 0) return err(PETSC_ERR_ARG_OUTOFRANGE, "dense matrix: negative size %d x %d", (int)m, (int)n);
+  if (!data) return err(PETSC_ERR_ARG_NULL, "dense matrix: null data array");
+  if (comm->size > 1) return err(PETSC_ERR_SUP, "dense matrices run on one rank (a %d-rank communicator was given)", comm->size);
+  if (dev) {
+    PB_CHK(dev_init());
+    PB_CHK(check_device_array(data, "dense matrix values"));
+  }
+  _p_Mat *A     = new _p_Mat;
+  A->comm       = comm;
+  A->kind       = MK_DENSE;
+  A->m = A->M   = m;
+  A->n = A->N   = n;
+  A->dn_src     = data;
+  A->dn_src_lda = m > 0 ? m : 1;
+  A->dn_src_dev = dev;
+  *mat          = A;
+  return 0;
+}
+PetscErrorCode MatCreateSeqDense(MPI_Comm comm, PetscInt m, PetscInt n, PetscScalar data[], Mat *A) { return dense_create(comm, m, n, data, false, A); }
+PetscErrorCode MatCreateSeqDenseCUDA(MPI_Comm comm, PetscInt m, PetscInt n, PetscScalar data[], Mat *A) { return dense_create(comm, m, n, data, true, A); }
+PetscErrorCode MatCreateDense(MPI_Comm comm, PetscInt m, PetscInt n, PetscInt M, PetscInt N, PetscScalar data[], Mat *A)
+{
+  if (comm->size > 1) return err(PETSC_ERR_SUP, "MatCreateDense: dense matrices run on one rank (a %d-rank communicator was given)", comm->size);
+  if (m == PETSC_DECIDE) m = M;
+  if (n == PETSC_DECIDE) n = N;
+  if ((M != PETSC_DECIDE && M != m) || (N != PETSC_DECIDE && N != n))
+    return err(PETSC_ERR_ARG_SIZ, "MatCreateDense: local size %d x %d differs from global %d x %d on one rank", (int)m, (int)n, (int)M, (int)N);
+  return dense_create(comm, m, n, data, false, A);
+}
+PetscErrorCode MatDenseSetLDA(Mat A, PetscInt lda)
+{
+  if (!A || A->kind != MK_DENSE) return err(PETSC_ERR_ARG_WRONG, "MatDenseSetLDA: dense matrix expected");
+  if (A->dn_ready) return err(PETSC_ERR_ARG_WRONGSTATE, "MatDenseSetLDA: the matrix has already been used");
+  if (lda < A->m || lda < 1) return err(PETSC_ERR_ARG_OUTOFRANGE, "MatDenseSetLDA: lda %d < %d rows", (int)lda, (int)A->m);
+  A->dn_src_lda = lda;
+  return 0;
+}
+PetscErrorCode MatDenseGetLDA(Mat A, PetscInt *lda)
+{
+  if (!A || A->kind != MK_DENSE) return err(PETSC_ERR_ARG_WRONG, "MatDenseGetLDA: dense matrix expected");
+  if (!lda) return err(PETSC_ERR_ARG_NULL, "null lda pointer");
+  *lda = (PetscInt)A->dn_src_lda;
+  return 0;
+}
+PetscErrorCode MatB200GetDenseInfo(Mat A, int64_t *lda, PetscBool *adopted, PetscInt *rows_per_block, PetscInt *split_columns)
+{
+  if (!A || A->kind != MK_DENSE) return err(PETSC_ERR_ARG_WRONG, "MatB200GetDenseInfo: dense matrix expected");
+  PB_CHK(pb::mat_ensure_device(A));
+  if (lda) *lda = A->Ad.dn_lda;
+  if (adopted) *adopted = A->dn_adopted ? PETSC_TRUE : PETSC_FALSE;
+  if (rows_per_block) *rows_per_block = A->Ad.dn_rpb;
+  if (split_columns) *split_columns = A->Ad.dn_split;
   return 0;
 }
 
@@ -1950,7 +2056,7 @@ PetscErrorCode MatCreateProd(MPI_Comm comm, PetscInt nmat, const Mat *mats, Mat 
   }
   Mat M2 = mats[0], M1 = mats[1];
   for (Mat F : {M1, M2})
-    if (F->kind != MK_AIJ && F->kind != MK_PROJ && F->kind != MK_PROD && F->kind != MK_PENALIZED) return err(PETSC_ERR_SUP, "MatCreateProd: unsupported factor kind");
+    if (F->kind != MK_AIJ && F->kind != MK_DENSE && F->kind != MK_PROJ && F->kind != MK_PROD && F->kind != MK_PENALIZED) return err(PETSC_ERR_SUP, "MatCreateProd: unsupported factor kind");
   // several GPUs: the factors are applied one after the other with their own halo exchanges / reductions (the un-fused route; the fused
   // MPGP driver takes product Hessians on one GPU only, qps.cpp: fused_eligible)
   if (M1->n != M2->m) return err(PETSC_ERR_ARG_SIZ, "MatCreateProd: inner dimensions differ (%d vs %d)", (int)M1->n, (int)M2->m);
@@ -2045,6 +2151,9 @@ int mat_mult_dev(Mat A, const double *x, double *y)
       PB_CHK(k_spmv(A->Ao, A->halo->d_ghost, y, 1));
     }
     return 0;
+  case MK_DENSE:
+    PB_CHK(mat_ensure_device(A));
+    return k_spmv(A->Ad, x, y, 0);
   case MK_PROD: {
     double *t;
     PB_CHK(vec_dev_write(A->twork, &t));
@@ -2205,9 +2314,9 @@ PetscErrorCode MatGetMaxEigenvalue(Mat A, Vec v, PetscReal *lambda_out, PetscRea
   if (tol == PETSC_DECIDE || tol == PETSC_DEFAULT) tol = 1e-4;            /* :473 */
   if (maxits == PETSC_DECIDE || maxits == PETSC_DEFAULT) maxits = 50;     /* :474 */
   // the reference looks for a stashed estimate first (:462-469); nothing in PERMON ever stores one, so there is none to return
-  if (!v && A->kind == MK_AIJ && A->comm->size == 1 && !getenv("PERMON_B200_NOFUSEDPOWER")) {
+  if (!v && (A->kind == MK_AIJ || A->kind == MK_DENSE) && A->comm->size == 1 && !getenv("PERMON_B200_NOFUSEDPOWER")) {
     PB_CHK(mat_ensure_device(A));
-    if ((A->Ad.kind == 3 || A->Ad.kind == 4) && A->m == A->n) {
+    if ((A->Ad.kind == 3 || A->Ad.kind == 4 || A->Ad.kind == 6) && A->m == A->n) {
       // fused form: one kernel per iteration (y = A (s w) with both dot products in its epilogue), the normalised iterate is never stored
       const PetscInt n = A->m;
       double        *w = nullptr, *y = nullptr;
